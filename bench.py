@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the GP-fitting hot path (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--n 20000]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--n 20000] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[1] -- Matern(nu=2.5), 3-D covariates, n = 20000, float64,
 one step = one evaluation of log marginal likelihood AND its gradient w.r.t. (log scale, log sigma_f, log sigma_n):
@@ -468,6 +468,30 @@ def measure_fp64_peaks(dev):
     return out
 
 
+DUMP_FACTOR_SAMPLES = 1 << 20
+
+
+def dump_outputs(path, last):
+    """ --dump-outputs: what the last timed evaluation computed, as float64 .npy files (8.5 MB at n = 20000): the
+    negative log marginal likelihood, its gradient w.r.t. (log ell, log sigma_f, log sigma_n), the diagonal of the
+    Cholesky factor L and a fixed seeded sample of 2^20 entries of its lower triangle (the whole of L is 3.2 GB) """
+    import torch
+    from lsqfitgp_b200 import _ops
+    st = last['st']
+    n = st.n
+    L = _ops.chol_get_factor(st)
+    rng = np.random.default_rng(6006)
+    i, j = rng.integers(0, n, (2, DUMP_FACTOR_SAMPLES))
+    flat = torch.as_tensor(np.maximum(i, j) * n + np.minimum(i, j), device=L.device)
+    arrays = dict(neg_logml=np.array([last['val']]), neg_logml_grad=last['grad'],
+                  chol_factor_diag=torch.diagonal(L).cpu().numpy(),
+                  chol_factor_sample=L.reshape(-1).index_select(0, flat).cpu().numpy())
+    del L
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), np.asarray(a, dtype=np.float64))
+
+
 def run_gpu(args):
     import torch
     import torch.distributed as dist
@@ -564,12 +588,15 @@ def run_gpu(args):
         return val, grad
 
     record_flag = [False]
+    last = {}   # --dump-outputs: the latest evaluation of the device arm (its factor stays alive until the next one)
 
     def fun_device(theta):
         """ unit of the sharded batch: (neg logML, gradient) of one hyperparameter point, device-resident inputs """
         ldq, vjp, st = step_device(theta, record=record_flag[0])
         assert int(st.info.item()) == 0
         val, grad = finish(theta, ldq, vjp)
+        if args.dump_outputs:
+            last.update(val=val, grad=grad, st=st)
         return np.r_[val, grad]
 
     # pinned host staging for the end-to-end arm
@@ -630,6 +657,9 @@ def run_gpu(args):
     assert out_dev.shape == (args.steps * world, 4) and np.all(np.isfinite(out_dev))
     phase_ms = {p: float(np.mean([ev[i].elapsed_time(ev[i + 1]) for ev in ev_log])) for i, p in enumerate(phases)}
     chol_inverse_span_ms = float(np.mean([ev[1].elapsed_time(ev[4]) for ev in ev_log]))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    last.clear()
 
     # ---- the Gram kernel alone (inside the step it is fused with the equilibration pass of the factorisation)
     gram_alone = []
@@ -930,7 +960,15 @@ def main():
     ap.add_argument('--c3-per-gpu', type=int, default=8, help='extra key c3_batch: points per GPU (0: skip)')
     ap.add_argument('--c1', type=int, default=1, help='extra key c1_latency at N = 1 (0: skip)')
     ap.add_argument('--c4', type=int, default=1, help='extra key c4_bart at N = 1 (0: skip)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last one computed as DIR/<name>.npy (float64, about '
+                         '8.5 MB): neg_logml, neg_logml_grad, chol_factor_diag, chol_factor_sample; the inputs depend on '
+                         'the arguments only, so two builds can be compared output for output')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs applies to the GPU arm (--impl ours)')
     if args.impl == 'reference':
         return run_reference(args)
     return run_gpu(args)

@@ -14,8 +14,7 @@ relative to the reference root).  The arithmetic lives in third-party code in th
   scipy >= 1.10: scipy.special.kv (called by the reference itself through pure_callback) -> same function.
 
 Pinning status (see tests/test_oracle_*.py, tests/golden/):
-  * fasthash64: pinned to the reference's 20 golden vectors (tests/test_jax.py:112-186) and to the
-    reference's own C source compiled into oracle/_ref (tests/fast-hash/fasthash.c).
+  * fasthash64: pinned to the reference's 20 golden vectors (tests/test_jax.py:112-186).
   * Chol: pinned by the reference's own test battery restated (tests/linalg/test_decomp.py:145-261:
     every method against scipy.linalg.solve / eigvalsh / finite differences).
   * Matern/Maternp cores: pinned by tests/test_special.py:68-97 restated (mpmath / scipy kv).

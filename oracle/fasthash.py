@@ -1,8 +1,5 @@
 """Oracle: fasthash64 (src/lsqfitgp/_jaxext/_fasthash.py:56-97 == tests/fast-hash/fasthash.c:34-66)."""
 
-import ctypes
-import pathlib
-
 import numpy as np
 
 M = 0x880355f21e6d1965
@@ -44,16 +41,3 @@ def fasthash64_rows(a, seed=BART_SEED):
     """ hash each row of a 2-d integer array over its raw bytes (as BART._correlation does on ix, iy) """
     a = np.ascontiguousarray(a)
     return np.array([fasthash64(row.tobytes(), seed) for row in a], dtype=np.uint64)
-
-
-def load_ref():
-    """ the reference's own C implementation compiled by oracle/Makefile into oracle/_ref (or None) """
-    p = pathlib.Path(__file__).resolve().parent / '_ref' / 'libfasthash_ref.so'
-    if not p.exists():
-        return None
-    lib = ctypes.CDLL(str(p))
-    lib.fasthash64.restype = ctypes.c_uint64
-    lib.fasthash64.argtypes = [ctypes.c_char_p, ctypes.c_size_t, ctypes.c_uint64]
-    lib.fasthash32.restype = ctypes.c_uint32
-    lib.fasthash32.argtypes = [ctypes.c_char_p, ctypes.c_size_t, ctypes.c_uint32]
-    return lib

@@ -6,8 +6,7 @@ for jax of oracle/refshim.py (jax, jaxlib and gvar are not installable in this i
 What runs is the reference's code: lgp.GP.marginal_likelihood / predfromdata(raw=True) (_GP/_compute.py), the kernel
 classes (_kernels/_basic.py, _matern.py, _bart.py with _Kernel/*), _linalg/_decomp.py Chol.  What stands in for JAX:
 numpy for jax.numpy, scipy LAPACK for jax.scipy.linalg, python loops for lax.scan / fori_loop.  tests/test_reference_vectors.py
-checks the oracle (and, on the GPU, the CUDA path) against the file, and regenerates it in memory when the reference tree
-is present to make sure the committed file is what this script produces."""
+checks the oracle (and, on the GPU, the CUDA path) against the file."""
 import pathlib
 import sys
 import warnings
