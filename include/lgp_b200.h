@@ -124,6 +124,31 @@ int lgp_gram_iso_jvp(lgp_stream_t stream, const lgp_factor_t *factors, int nfact
                      int64_t ldx, int64_t n, const double *y, int64_t ldy, int64_t m, const double *tangent,
                      double *D_out, int64_t ldd);
 
+/* Derivative blocks: the covariance between first derivatives of the process, cov(d f(x)/d x_a, d f(y)/d y_b), with
+ * a = dx_field, b = dy_field (field indices; -1 = no derivative on that argument, both -1 is LGP_ERR_BADARG).
+ * Replaces the reference's jax derivatives of the kernel core behind addx(deriv=) and CrossKernel.linop('diff')
+ * (src/lsqfitgp/_GP/_elements.py:190-242, _Kernel/_crosskernel.py:281-347, _Kernel/_ops.py:200-290):
+ *   K[i][j] = d/dx_a d/dy_b k(x_i, y_j)   (only the derivatives requested),
+ * the derivatives taken with respect to the raw coordinates (1/scale chain factors included).  Only first derivatives;
+ * a factor that depends on a differentiated field must be ExpQuad, Maternp with p >= 1 or Cauchy with alpha = 2
+ * (otherwise LGP_ERR_UNSUPPORTED); the other factors may be of any kind.  Same layouts as lgp_gram_iso;
+ * flags: LGP_GRAM_SYMMETRIC with x == y and dx_field == dy_field evaluates the lower tiles once and mirrors them. */
+int lgp_gram_iso_deriv(lgp_stream_t stream, const lgp_factor_t *factors, int nfactors, int ndim, const double *x,
+                       int64_t ldx, int64_t n, const double *y, int64_t ldy, int64_t m, int dx_field, int dy_field,
+                       double *K_out, int64_t ldk, int flags);
+
+/* Reverse-mode contraction of a derivative block (dense G, n x m, ldg), the out layout of lgp_gram_iso_vjp:
+ * out[3f+k] = sum_ij G_ij d K_ij / d(amp_f, log scale_f, par1_f).  out: device, 3*nfactors doubles (zeroed by the call;
+ * atomicAdd accumulation). */
+int lgp_gram_iso_deriv_vjp(lgp_stream_t stream, const lgp_factor_t *factors, int nfactors, int ndim, const double *x,
+                           int64_t ldx, int64_t n, const double *y, int64_t ldy, int64_t m, int dx_field, int dy_field,
+                           const double *G, int64_t ldg, double *out);
+
+/* Forward-mode derivative of a derivative block along `tangent` (HOST, 3*nfactors doubles, layout of lgp_gram_iso_jvp). */
+int lgp_gram_iso_deriv_jvp(lgp_stream_t stream, const lgp_factor_t *factors, int nfactors, int ndim, const double *x,
+                           int64_t ldx, int64_t n, const double *y, int64_t ldy, int64_t m, int dx_field, int dy_field,
+                           const double *tangent, double *D_out, int64_t ldd);
+
 /* Variants with DEVICE-RESIDENT hyperparameters: what an XLA-FFI custom call needs, where traced scalars arrive as device
  * buffers and must not be read on the host (the boundary B3 of SURVEY.md section 8b: jax.ffi handlers wrapping these are in
  * lsqfitgp_b200/csrc/xla_ffi_shim.cc, INTEGRATION.md section 3).  `factors` (HOST) carries only the structure: kind, term,

@@ -24,6 +24,7 @@ import torch
 
 from . import _array
 from . import _Kernel
+from ._Deriv import Deriv
 from . import _lib
 from . import _linalg
 from . import _ops
@@ -59,10 +60,17 @@ class _Element:
 
 
 class _Points(_Element):
-    def __init__(self, labels, xd, shape):
+    def __init__(self, labels, xd, shape, deriv=None, dfield=-1):
         self.labels = labels
         self.xd = xd          # (ndim, n) float64 device tensor
         self.shape = shape
+        self.deriv = Deriv(deriv)
+        self.dfield = dfield  # index of the differentiated field in labels, -1: the process itself
+
+
+def _plain_points(elem):
+    """ points of the process itself (no derivative): what the fused single-key fast paths handle """
+    return isinstance(elem, _Points) and elem.dfield < 0
 
 
 class _LinTransf(_Element):
@@ -89,19 +97,23 @@ class _GramFn(torch.autograd.Function):
     Gram build, src/lsqfitgp/_fit.py:687-702). """
 
     @staticmethod
-    def forward(ctx, kern, xd, yd, labels, *params):
-        ctx.kern, ctx.xd, ctx.yd, ctx.labels = kern, xd, yd, labels
-        return kern._gram_device(xd, yd, labels, symmetric=xd is yd)
+    def forward(ctx, kern, xd, yd, labels, dfields, *params):
+        ctx.kern, ctx.xd, ctx.yd, ctx.labels, ctx.dfields = kern, xd, yd, labels, dfields
+        return kern._gram_device(xd, yd, labels, symmetric=xd is yd, dfields=dfields)
 
     @staticmethod
     def backward(ctx, G):
-        kern, xd, yd, labels = ctx.kern, ctx.xd, ctx.yd, ctx.labels
+        kern, xd, yd, labels, dfields = ctx.kern, ctx.xd, ctx.yd, ctx.labels, ctx.dfields
         hyper = kern._hyperparams()
         grads = []
         vjp = None
         if kern._terms:
             descs, index = kern._descriptor(labels)
-            vjp = _ops.gram_iso_vjp_general(descs, xd, yd, _ops.as_aligned(G.contiguous())).cpu()
+            Ga = _ops.as_aligned(G.contiguous())
+            if dfields != (-1, -1):
+                vjp = _ops.gram_iso_deriv_vjp(descs, xd, yd, dfields[0], dfields[1], Ga).cpu()
+            else:
+                vjp = _ops.gram_iso_vjp_general(descs, xd, yd, Ga).cpu()
             pos = {tf: i for i, tf in enumerate(index)}
         bart_vjp = {}  # one fused pass per BART term: [d/d amp, d/d alpha, d/d beta]
         for kind, ti, fi, tensor in hyper:
@@ -119,13 +131,13 @@ class _GramFn(torch.autograd.Function):
             else:  # pragma: no cover
                 raise NotImplementedError(kind)
             grads.append(g.to(tensor.device, tensor.dtype).reshape(tensor.shape))
-        return (None, None, None, None, *grads)
+        return (None, None, None, None, None, *grads)
 
     @staticmethod
-    def jvp(ctx, _kern, _xd, _yd, _labels, *tangents):
+    def jvp(ctx, _kern, _xd, _yd, _labels, _dfields, *tangents):
         """ forward mode (torch.autograd.forward_ad): dK along the tangent of the hyperparameters, one pass of
         lgp_gram_iso_jvp; what jax.jacfwd of the Gram build gives the reference's Fisher path (_fit.py:676-683) """
-        kern, xd, yd, labels = ctx.kern, ctx.xd, ctx.yd, ctx.labels
+        kern, xd, yd, labels, dfields = ctx.kern, ctx.xd, ctx.yd, ctx.labels, ctx.dfields
         hyper = kern._hyperparams()
         assert len(hyper) == len(tangents)
         D = None
@@ -145,7 +157,10 @@ class _GramFn(torch.autograd.Function):
                     tan[pos[(ti, fi)], 2] += tv
                 else:  # pragma: no cover
                     raise NotImplementedError(kind)
-            D = _ops.gram_iso_jvp(descs, xd, yd, tan)
+            if dfields != (-1, -1):
+                D = _ops.gram_iso_deriv_jvp(descs, xd, yd, dfields[0], dfields[1], tan)
+            else:
+                D = _ops.gram_iso_jvp(descs, xd, yd, tan)
         # BART terms: D += t_amp corr + t_alpha amp dcorr/dalpha + t_beta amp dcorr/dbeta, one kernel pass per term
         bart_tan = {}
         for (kind, ti, fi, tensor), t in zip(hyper, tangents):
@@ -318,9 +333,9 @@ class GP:
     # ------------------------------------------------------------------------------------------------
     @_newself
     def addx(self, x, key=None, *, deriv=0, proc=None):
-        """ Add points where the Gaussian process is evaluated (reference _elements.py:158-242) """
-        if deriv not in (0, None) and deriv != {}:
-            raise NotImplementedError('derivatives of the process')
+        """ Add points where the Gaussian process is evaluated (reference _elements.py:158-242).
+        `deriv` (see `Deriv`): the points are of the first derivative of the process w.r.t. that field (order <= 1). """
+        deriv = Deriv(deriv)
         if proc is not None:
             raise NotImplementedError('multiple processes')
         if self._covfun is None:
@@ -342,9 +357,11 @@ class GP:
             names = tuple(labels)
             if self._dtype_names is not None and self._dtype_names != names:
                 raise TypeError(f'x[{key!r}] has fields {names!r} not compatible with {self._dtype_names!r}')
+            dfield = _Kernel.deriv_field(deriv, labels) if deriv.order <= 1 else None
+            self._covfun._check_derivable(deriv, 0)
             self._dtype_names = names
             xd = torch.from_numpy(numpy.ascontiguousarray(data)).to(dev)
-            self._elements[key] = _Points(labels, xd, tuple(shape))
+            self._elements[key] = _Points(labels, xd, tuple(shape), deriv, dfield)
 
     @_newself
     def addcov(self, covblocks, key=None, *, decomps=None):
@@ -508,13 +525,14 @@ class GP:
         y = self._elements[ykey]
         kern = self._covfun
         yd = x.xd if y is x else y.xd
+        dfields = (x.dfield, y.dfield)
         if self._grad_mode():
             params = [h[3] for h in kern._hyperparams()]
-            cov = _GramFn.apply(kern, x.xd, yd, x.labels, *params)
+            cov = _GramFn.apply(kern, x.xd, yd, x.labels, dfields, *params)
             if out is not None:
                 raise RuntimeError('internal: out= in grad mode')
             return cov
-        return kern._gram_device(x.xd, yd, x.labels, out=out, symmetric=y is x)
+        return kern._gram_device(x.xd, yd, x.labels, out=out, symmetric=y is x, dfields=dfields)
 
     def _makecovblock_lintransf_any(self, xkey, ykey):
         x = self._elements[xkey]
@@ -689,7 +707,7 @@ class GP:
             if cache is not None:
                 return cache
         if (hasattr(self._decompbase, 'from_kernel') and len(keys) == 1 and ycov is None and not covtransf
-                and isinstance(self._elements[keys[0]], _Points) and self._covfun._terms and not self._covfun._bart
+                and _plain_points(self._elements[keys[0]]) and self._covfun._terms and not self._covfun._bart
                 and (keys[0], keys[0]) not in self._covblocks):
             # distributed solver on one set of points with a kernel-only covariance: every rank generates its own tiles
             # from the replicated points; the n x n matrix is never assembled (the case that outgrows one GPU)
@@ -703,7 +721,7 @@ class GP:
             self._decompcache[keys] = decomp
             return decomp
         if (self._solver_name == 'chol' and len(keys) == 1 and ycov is None and not covtransf
-                and isinstance(self._elements[keys[0]], _Points) and self._covfun is not None and self._covfun._terms
+                and _plain_points(self._elements[keys[0]]) and self._covfun is not None and self._covfun._terms
                 and not self._covfun._bart and (keys[0], keys[0]) not in self._covblocks and not self._grad_mode()):
             # one set of points, kernel-only covariance, matrix not built yet: Gram build fused with the equilibration pass
             # of the factorisation (lgp_gram_iso_prepare), for the kernels of the fast family.  The finiteness check of the
@@ -928,7 +946,7 @@ class GP:
                                       "distributed decomposition is value-only, use solver='chol' for gradients")
         solverkw = dict(self._solverkw)
         solverkw.update(kw)
-        if (len(inkeys) == 1 and ycov is None and isinstance(self._elements[inkeys[0]], _Points)
+        if (len(inkeys) == 1 and ycov is None and _plain_points(self._elements[inkeys[0]])
                 and self._covfun._terms and not self._covfun._bart):
             elem = self._elements[inkeys[0]]
             params = [h[3] for h in self._covfun._hyperparams()]

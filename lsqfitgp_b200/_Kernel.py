@@ -20,6 +20,7 @@ import numpy
 import torch
 
 from . import _array
+from ._Deriv import Deriv
 from . import _lib
 from . import _ops
 
@@ -57,10 +58,12 @@ def _pair(arg):
 class _Factor:
     """ one isotropic factor: core(kind, params) applied to r2 over selected fields after loc/scale """
 
-    __slots__ = ('kind', 'ipar', 'par0', 'par1', 'scale', 'loc', 'dim')
+    __slots__ = ('kind', 'ipar', 'par0', 'par1', 'scale', 'loc', 'dim', 'derivable')
 
-    def __init__(self, kind, ipar=0, par0=0.0, par1=0.0, scale=(None, None), loc=(None, None), dim=(None, None)):
+    def __init__(self, kind, ipar=0, par0=0.0, par1=0.0, scale=(None, None), loc=(None, None), dim=(None, None),
+                 derivable=0):
         self.kind = kind
+        self.derivable = derivable   # how many times the factor may be differentiated w.r.t. each of its fields
         self.ipar = ipar
         self.par0 = par0
         self.par1 = par1
@@ -69,7 +72,7 @@ class _Factor:
         self.dim = dim
 
     def replace(self, **kw):
-        new = _Factor(self.kind, self.ipar, self.par0, self.par1, self.scale, self.loc, self.dim)
+        new = _Factor(self.kind, self.ipar, self.par0, self.par1, self.scale, self.loc, self.dim, self.derivable)
         for k, v in kw.items():
             setattr(new, k, v)
         return new
@@ -91,6 +94,7 @@ class CrossKernel:
 
     _kind = None          # set by concrete kernels (_kernels.py)
     _derivable = None
+    _diff = None          # (Deriv of x, Deriv of y) of a kernel made by linop('diff')
 
     def __new__(cls, *args, **kw):
         if cls._kind is None and (args or kw):
@@ -101,6 +105,7 @@ class CrossKernel:
         self = object.__new__(cls)
         self._terms = ()
         self._bart = ()
+        self._diff = None
         return self
 
     # ---- construction helpers used by _kernels.py
@@ -122,9 +127,10 @@ class CrossKernel:
         for d in (dx, dy):
             if d is not None and not isinstance(d, (str, list)):
                 raise TypeError(f'dim must be a (list of) string, found {d!r}')
-        fac = _Factor(kind, ipar, par0, par1, (sx, sy), (lx, ly), (dx, dy))
+        fac = _Factor(kind, ipar, par0, par1, (sx, sy), (lx, ly), (dx, dy), 0 if derivable is None else derivable)
         self._terms = (_Term(1.0, (fac,)),)
         self._bart = ()
+        self._diff = None
         self._maxdim = maxdim
         return self
 
@@ -132,12 +138,14 @@ class CrossKernel:
         new = object.__new__(cls or type(self))
         new._terms = self._terms if terms is None else tuple(terms)
         new._bart = self._bart if bart is None else tuple(bart)
+        new._diff = None
         return new
 
     # ---- algebra (reference: _Kernel/_alg.py:32-143, _crosskernel.py:235-249)
     def __add__(self, other):
+        _no_algebra_on_diff(self, other)
         if _isscalar(other):
-            const = _Term(other, (_Factor(_lib.K_CONSTANT),))
+            const = _Term(other, (_Factor(_lib.K_CONSTANT, derivable=numpy.inf),))
             return self._clone(_common_class(type(self), IsotropicKernel), terms=self._terms + (const,))
         if isinstance(other, CrossKernel):
             return self._clone(_common_class(type(self), type(other)), terms=self._terms + other._terms,
@@ -147,6 +155,7 @@ class CrossKernel:
     __radd__ = __add__
 
     def __mul__(self, other):
+        _no_algebra_on_diff(self, other)
         if _isscalar(other):
             terms = [_Term(_mulamp(t.amp, other), t.factors) for t in self._terms]
             bart = [b.scaled(other) for b in self._bart]
@@ -183,10 +192,12 @@ class CrossKernel:
             args = args * 2
         if all(a is None for a in args):
             return self
+        if transfname == 'diff':
+            return self._linop_diff(*args)
         if transfname not in ('scale', 'loc', 'dim'):
-            if transfname == 'diff' and all(not a for a in args):
-                return self
             raise NotImplementedError(f'linop {transfname!r}')
+        if self._diff is not None:
+            raise NotImplementedError(f'linop {transfname!r} after linop(\'diff\')')
         if self._bart:
             raise NotImplementedError(f'linop {transfname!r} on the BART kernel')
         terms = []
@@ -199,6 +210,45 @@ class CrossKernel:
                 facs.append(f.replace(**{transfname: tuple(args)}))
             terms.append(_Term(t.amp, facs))
         return self._clone(terms=terms)
+
+    def _linop_diff(self, dx, dy):
+        """ k(x, y) -> d/dx_a d/dy_b k(x, y) for derivatives of order <= 1 on each argument (reference
+        _Kernel/_crosskernel.py linop('diff') and _Kernel/_ops.py, Diff) """
+        dx, dy = Deriv(dx), Deriv(dy)
+        if not dx and not dy:
+            return self
+        if self._diff is not None:
+            raise NotImplementedError("composition of two 'diff' transformations")
+        self._check_derivable(dx, 0)
+        self._check_derivable(dy, 1)
+        new = self._clone(CrossKernel)
+        new._diff = (dx, dy)
+        return new
+
+    def _check_derivable(self, deriv, side):
+        """ ValueError if the derivative `deriv` of argument `side` (0 = x, 1 = y) exceeds the derivability of a factor
+        that depends on its field (factors that do not depend on it impose no limit); NotImplementedError for what the
+        kernels cannot compute (order > 1 on one argument, Matern of non-half-integer order) """
+        if not deriv:
+            return
+        for field, order in deriv:
+            for t in self._terms:
+                for f in t.factors:
+                    if not _factor_depends_on(f, field, side):
+                        continue
+                    if order > f.derivable:
+                        raise ValueError(f'derivative of order {order} w.r.t. {field!r} exceeds the derivability '
+                                         f'{f.derivable} of the kernel')
+            if self._bart:
+                raise ValueError(f'derivative of order {order} w.r.t. {field!r} exceeds the derivability 0 of the '
+                                 'BART kernel')
+        if deriv.order > 1:
+            raise NotImplementedError(f'derivative of order {deriv.order} > 1 on one argument')
+        for field, order in deriv:
+            for t in self._terms:
+                for f in t.factors:
+                    if f.kind == _lib.K_MATERN and _factor_depends_on(f, field, side):
+                        raise NotImplementedError('derivatives of Matern of non-half-integer order')
 
     def batch(self, maxnbytes):
         """ the reference chunks the evaluation to bound temporaries (_jaxext/_batcher.py); the fused kernel has none """
@@ -213,10 +263,13 @@ class CrossKernel:
         if lx != ly:
             raise ValueError(f'x and y have different fields: {lx} vs {ly}')
         shape = numpy.broadcast_shapes(sx, sy)
+        dfields = None
+        if self._diff is not None:
+            dfields = (deriv_field(self._diff[0], lx), deriv_field(self._diff[1], ly))
         dev = torch.device('cuda', torch.cuda.current_device())
         xd = torch.from_numpy(numpy.ascontiguousarray(cx)).to(dev)
         yd = torch.from_numpy(numpy.ascontiguousarray(cy)).to(dev)
-        G = self._gram_device(xd, yd, lx).cpu().numpy()
+        G = self._gram_device(xd, yd, lx, dfields=dfields).cpu().numpy()
         ix = numpy.broadcast_to(numpy.arange(cx.shape[1]).reshape(sx), shape)
         iy = numpy.broadcast_to(numpy.arange(cy.shape[1]).reshape(sy), shape)
         return G[ix, iy]
@@ -245,11 +298,20 @@ class CrossKernel:
             raise NotImplementedError(f'kernel expression has {len(descs)} factors > {_lib.MAX_FACTORS}')
         return descs, index
 
-    def _gram_device(self, xd, yd, labels, out=None, symmetric=False):
-        """ Gram matrix on the device. xd: (ndim, n), yd: (ndim, m) float64 cuda tensors """
+    def _gram_device(self, xd, yd, labels, out=None, symmetric=False, dfields=None):
+        """ Gram matrix on the device. xd: (ndim, n), yd: (ndim, m) float64 cuda tensors; dfields: (a, b) field
+        indices of a derivative block d/dx_a d/dy_b (-1: none on that argument), see deriv_field """
         n, m = xd.shape[1], yd.shape[1]
         if out is None:
             out = _ops.aligned_empty(n, m, xd.device)
+        if dfields is not None and dfields != (-1, -1):
+            assert not self._bart   # rejected by _check_derivable
+            if self._terms:
+                descs, _ = self._descriptor(labels)
+                _ops.gram_iso_deriv(descs, xd, yd, dfields[0], dfields[1], out=out, symmetric=symmetric)
+            else:
+                out.zero_()
+            return out
         have = False
         if self._terms:
             descs, _ = self._descriptor(labels)
@@ -289,6 +351,45 @@ class CrossKernel:
         for b in self._bart:
             out += b.hyperparams()
         return out
+
+
+def _no_algebra_on_diff(a, b):
+    if getattr(a, '_diff', None) is not None or getattr(b, '_diff', None) is not None:
+        raise NotImplementedError("algebra on a kernel transformed by linop('diff')")
+
+
+def _factor_depends_on(f, field, side):
+    """ whether factor f depends on `field` (None: the coordinate of unstructured points) of argument `side` """
+    if f.kind == _lib.K_CONSTANT:
+        return False
+    dim = f.dim[side]
+    if dim is None or field is None:
+        return True
+    return field in ([dim] if isinstance(dim, str) else dim)
+
+
+def deriv_field(deriv, labels):
+    """ index into `labels` of the field of a first-order derivative, -1 for no derivative """
+    deriv = Deriv(deriv)
+    if not deriv:
+        return -1
+    if labels == [None]:
+        if not deriv.implicit:
+            raise ValueError(f'derivative {deriv!r} w.r.t. named fields of non-structured points')
+        return 0
+    if deriv.implicit:
+        raise ValueError(f'implicit derivative {deriv!r} of structured points: name the field')
+    out = []
+    for field, _ in deriv:
+        idx = [i for i, lab in enumerate(labels) if (lab[0] if isinstance(lab, tuple) else lab) == field]
+        if not idx:
+            raise ValueError(f'derivative field {field!r} not in x')
+        if len(idx) != 1 or isinstance(labels[idx[0]], tuple):
+            raise NotImplementedError(f'derivative w.r.t. {field!r}, which is not a single scalar field')
+        out.append(idx[0])
+    if len(out) != 1 or deriv.order != 1:
+        raise NotImplementedError(f'derivative {deriv!r} of order > 1 on one argument')
+    return out[0]
 
 
 def _mulamp(a, b):

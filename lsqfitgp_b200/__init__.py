@@ -9,6 +9,7 @@ __version__ = '0.1.0'
 
 from . import _lib  # noqa: F401
 from ._array import StructuredArray, unstructured_to_structured, asarray
+from ._Deriv import Deriv
 from ._Kernel import (CrossKernel, Kernel, CrossStationaryKernel, StationaryKernel, CrossIsotropicKernel,
                       IsotropicKernel, kernel, stationarykernel, isotropickernel, crosskernel,
                       crossstationarykernel, crossisotropickernel)

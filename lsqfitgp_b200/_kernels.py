@@ -21,7 +21,7 @@ class Constant(IsotropicKernel):
     _kind = _lib.K_CONSTANT
 
     def __new__(cls, **kw):
-        return cls._make(cls._kind, **kw)
+        return cls._make(cls._kind, derivable=numpy.inf, **kw)
 
 
 class White(IsotropicKernel):
@@ -37,7 +37,7 @@ class ExpQuad(IsotropicKernel):
     _kind = _lib.K_EXPQUAD
 
     def __new__(cls, **kw):
-        return cls._make(cls._kind, **kw)
+        return cls._make(cls._kind, derivable=numpy.inf, **kw)
 
 
 class Cauchy(IsotropicKernel):
@@ -47,7 +47,7 @@ class Cauchy(IsotropicKernel):
     def __new__(cls, alpha=2, beta=2, **kw):
         assert 0 < _f(alpha) <= 2, alpha
         assert 0 < _f(beta), beta
-        return cls._make(cls._kind, par0=alpha, par1=beta, **kw)
+        return cls._make(cls._kind, par0=alpha, par1=beta, derivable=numpy.inf if _f(alpha) == 2 else 0, **kw)
 
 
 class Maternp(IsotropicKernel):
@@ -56,7 +56,7 @@ class Maternp(IsotropicKernel):
 
     def __new__(cls, p=None, **kw):
         assert p is not None and int(p) == p and p >= 0, p
-        return cls._make(cls._kind, ipar=int(p), par0=1e-30, **kw)
+        return cls._make(cls._kind, ipar=int(p), par0=1e-30, derivable=int(p), **kw)
 
 
 class Matern(IsotropicKernel):
@@ -75,10 +75,10 @@ class Matern(IsotropicKernel):
             raise NotImplementedError('Matern: derivatives with respect to nu are not implemented (nor in the reference)')
         p = _f(nu) - 0.5
         if p >= 0 and p == int(p) and p <= 8:
-            return cls._make(_lib.K_MATERNP, ipar=int(p), par0=0.0, **kw)
+            return cls._make(_lib.K_MATERNP, ipar=int(p), par0=0.0, derivable=int(p), **kw)
         if _f(nu) > 100:
             raise NotImplementedError(f'Matern(nu={nu!r}): orders above 100 are not implemented on the device')
-        return cls._make(_lib.K_MATERN, par0=_f(nu), **kw)
+        return cls._make(_lib.K_MATERN, par0=_f(nu), derivable=max(0, int(numpy.ceil(_f(nu))) - 1), **kw)
 
 
 # -------------------------------------------------------------------------------------------------

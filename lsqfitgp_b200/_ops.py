@@ -141,6 +141,57 @@ def gram_iso_jvp(descs, x, y, tangent, out=None):
     return out
 
 
+def gram_iso_deriv(descs, x, y, dx_field, dy_field, out=None, symmetric=False):
+    """ derivative block d/dx_a d/dy_b k(x, y) (lgp_gram_iso_deriv): a = dx_field, b = dy_field field indices, -1 for
+    no derivative on that argument; otherwise as gram_iso """
+    lib = _lib.load()
+    ndim, n = x.shape
+    m = y.shape[1]
+    x = x.contiguous() if x.stride(1) != 1 else x
+    y = y.contiguous() if y.stride(1) != 1 else y
+    if out is None:
+        out = aligned_empty(n, m, x.device)
+    facs = make_factors(descs)
+    check(lib.lgp_gram_iso_deriv(stream_ptr(), facs, len(descs), ndim, ptr(x), x.stride(0), n, ptr(y), y.stride(0), m,
+                                 int(dx_field), int(dy_field), ptr(out), out.stride(0), 1 if symmetric else 0),
+          'lgp_gram_iso_deriv')
+    return out
+
+
+def gram_iso_deriv_vjp(descs, x, y, dx_field, dy_field, G):
+    """ (nfactors, 3) device tensor: sum_ij G_ij d block_ij / d(amp, log scale, par1), G dense (n, m) """
+    lib = _lib.load()
+    ndim, n = x.shape
+    m = y.shape[1]
+    x = x.contiguous() if x.stride(1) != 1 else x
+    y = y.contiguous() if y.stride(1) != 1 else y
+    assert G.shape == (n, m) and G.stride(1) == 1
+    buf = torch.empty(3 * len(descs), dtype=f64, device=x.device)
+    facs = make_factors(descs)
+    check(lib.lgp_gram_iso_deriv_vjp(stream_ptr(), facs, len(descs), ndim, ptr(x), x.stride(0), n, ptr(y), y.stride(0),
+                                     m, int(dx_field), int(dy_field), ptr(G), G.stride(0), ptr(buf)),
+          'lgp_gram_iso_deriv_vjp')
+    return buf.reshape(len(descs), 3)
+
+
+def gram_iso_deriv_jvp(descs, x, y, dx_field, dy_field, tangent, out=None):
+    """ forward-mode derivative of the derivative block along `tangent` (layout of gram_iso_jvp) """
+    lib = _lib.load()
+    ndim, n = x.shape
+    m = y.shape[1]
+    x = x.contiguous() if x.stride(1) != 1 else x
+    y = y.contiguous() if y.stride(1) != 1 else y
+    if out is None:
+        out = aligned_empty(n, m, x.device)
+    tan = numpy.ascontiguousarray(numpy.asarray(tangent, dtype=numpy.float64).reshape(-1))
+    assert tan.size == 3 * len(descs)
+    facs = make_factors(descs)
+    check(lib.lgp_gram_iso_deriv_jvp(stream_ptr(), facs, len(descs), ndim, ptr(x), x.stride(0), n, ptr(y), y.stride(0),
+                                     m, int(dx_field), int(dy_field), tan.ctypes.data_as(_lib.c_double_p), ptr(out),
+                                     out.stride(0)), 'lgp_gram_iso_deriv_jvp')
+    return out
+
+
 def devpar_of(descs, device):
     """ (nfactors, 6) device tensor of the numeric descriptor fields in the LGP_DEVPAR_STRIDE order
     (scale_x, scale_y, loc_x, loc_y, par1, amp): what a traced caller keeps on the device """
