@@ -25,6 +25,24 @@ namespace lgp { void count_launch(); }
 
 namespace lgp {
 
+// Opt `kernel` in to `dyn` bytes of dynamic shared memory before a launch.  Without the opt-in a launch may use 48 KiB
+// of static plus dynamic shared memory in all; so the kernel's static size counts against that limit too.  A failed
+// query or opt-in is cleared from cudaGetLastError so that it does not surface at a later, unrelated launch check.
+template <class F>
+static int smem_opt_in(F *kernel, size_t dyn) {
+    cudaFuncAttributes fa;
+    if (cudaFuncGetAttributes(&fa, (const void *)kernel) != cudaSuccess) {
+        cudaGetLastError();
+        return LGP_ERR_CUDA;
+    }
+    if (fa.sharedSizeBytes + dyn <= 48 * 1024) return LGP_OK;
+    if (cudaFuncSetAttribute((const void *)kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn) != cudaSuccess) {
+        cudaGetLastError();
+        return LGP_ERR_CUDA;
+    }
+    return LGP_OK;
+}
+
 __device__ __forceinline__ uint32_t smem_u32(const void *p) {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));
 }

@@ -279,12 +279,6 @@ static int build_deriv(const lgp_factor_t *f, int nf, int ndim, int dx_field, in
     return LGP_OK;
 }
 
-static int deriv_smem_attr(const void *kernel, size_t smem) {
-    if (smem > 48 * 1024 && cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-        return LGP_ERR_CUDA;
-    return LGP_OK;
-}
-
 static int deriv_launch(lgp_stream_t stream, const lgp_factor_t *factors, int nfactors, int ndim, const double *x,
                         int64_t ldx, int64_t n, const double *y, int64_t ldy, int64_t m, int dx_field, int dy_field,
                         const double *tangent, double *K_out, int64_t ldk, int flags) {
@@ -311,11 +305,11 @@ static int deriv_launch(lgp_stream_t stream, const lgp_factor_t *factors, int nf
     const size_t smem = (size_t)2 * d.nslots * GT * sizeof(double) + (sym ? (size_t)GT * (GT + 1) * sizeof(double) : 0);
     cudaStream_t st = (cudaStream_t)stream;
     if (tangent) {
-        if (deriv_smem_attr((const void *)gram_deriv_kernel<true>, smem)) return LGP_ERR_CUDA;
+        if (smem_opt_in(gram_deriv_kernel<true>, smem)) return LGP_ERR_CUDA;
         gram_deriv_kernel<true><<<(unsigned)nblk, G_THREADS, smem, st>>>(d, ds, tan, x, ldx, n, y, ldy, m, K_out, ldk, 0,
                                                                          (int)tn);
     } else {
-        if (deriv_smem_attr((const void *)gram_deriv_kernel<false>, smem)) return LGP_ERR_CUDA;
+        if (smem_opt_in(gram_deriv_kernel<false>, smem)) return LGP_ERR_CUDA;
         gram_deriv_kernel<false><<<(unsigned)nblk, G_THREADS, smem, st>>>(d, ds, tan, x, ldx, n, y, ldy, m, K_out, ldk,
                                                                           sym ? 1 : 0, (int)tn);
     }
@@ -358,7 +352,7 @@ int lgp_gram_iso_deriv_vjp(lgp_stream_t stream, const lgp_factor_t *factors, int
     const int64_t tm = (n + GT - 1) / GT, tn = (m + GT - 1) / GT;
     if (tm * tn > 2147483647LL) return LGP_ERR_UNSUPPORTED;
     const size_t smem = (size_t)2 * d.nslots * GT * sizeof(double);
-    if (deriv_smem_attr((const void *)gram_deriv_vjp_kernel, smem)) return LGP_ERR_CUDA;
+    if (smem_opt_in(gram_deriv_vjp_kernel, smem)) return LGP_ERR_CUDA;
     gram_deriv_vjp_kernel<<<(unsigned)(tm * tn), G_THREADS, smem, st>>>(d, ds, x, ldx, n, y, ldy, m, G, ldg, (int)tn, out);
     LGP_CUDA_CHECK_LAUNCH();
     return LGP_OK;

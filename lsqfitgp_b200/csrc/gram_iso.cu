@@ -1361,13 +1361,11 @@ static int launch_fast(cudaStream_t st, const FastDesc &d, const double *x, int6
     if (grid > 2147483647LL) return LGP_ERR_UNSUPPORTED;
     int vec_ok = ((ldk & 1) == 0) && ((reinterpret_cast<uintptr_t>(K) & 15) == 0);
     if (sym) {
-        if (smem > 48 * 1024)
-            cudaFuncSetAttribute(gram_fast_kernel<KIND, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (smem_opt_in(gram_fast_kernel<KIND, true>, smem)) return LGP_ERR_CUDA;
         gram_fast_kernel<KIND, true><<<(unsigned)grid, G_THREADS, smem, st>>>(d, x, ldx, n, y, ldy, m, K, ldk, vec_ok,
                                                                              (int)tn);
     } else {
-        if (smem > 48 * 1024)
-            cudaFuncSetAttribute(gram_fast_kernel<KIND, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (smem_opt_in(gram_fast_kernel<KIND, false>, smem)) return LGP_ERR_CUDA;
         gram_fast_kernel<KIND, false><<<(unsigned)grid, G_THREADS, smem, st>>>(d, x, ldx, n, y, ldy, m, K, ldk, vec_ok,
                                                                               (int)tn);
     }
@@ -1416,13 +1414,11 @@ static int launch_fast2(cudaStream_t st, const FastDesc &d, const double *x, int
         gram_fast3_kernel<KIND, P, 3, false><<<g3, G_THREADS, smem, st>>>(d, x, ldx, n, K, ldk, vec_ok, (long long)grid,
                                                                           GramPrep{nullptr, nullptr, 0});
     } else if (sym) {
-        if (smem > 48 * 1024)
-            cudaFuncSetAttribute(gram_fast2_kernel<KIND, P, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (smem_opt_in(gram_fast2_kernel<KIND, P, true>, smem)) return LGP_ERR_CUDA;
         gram_fast2_kernel<KIND, P, true><<<(unsigned)grid, G_THREADS, smem, st>>>(d, x, ldx, n, y, ldy, m, K, ldk,
                                                                                  vec_ok, (int)tn);
     } else {
-        if (smem > 48 * 1024)
-            cudaFuncSetAttribute(gram_fast2_kernel<KIND, P, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (smem_opt_in(gram_fast2_kernel<KIND, P, false>, smem)) return LGP_ERR_CUDA;
         gram_fast2_kernel<KIND, P, false><<<(unsigned)grid, G_THREADS, smem, st>>>(d, x, ldx, n, y, ldy, m, K, ldk,
                                                                                   vec_ok, (int)tn);
     }
@@ -1560,13 +1556,6 @@ __global__ void zero_kernel(double *p, int n) {
 
 // ---- launchers of the general kernels: numeric descriptor fields from the host struct (devpar == nullptr) or from
 // device memory (the *_dev entry points)
-template <class F>
-static int general_smem_attr(F kernel, size_t smem) {
-    if (smem > 48 * 1024 &&
-        cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-        return LGP_ERR_CUDA;
-    return LGP_OK;
-}
 
 static int gram_general(lgp_stream_t stream, const lgp_factor_t *factors, int nfactors, int ndim, const double *devpar,
                         const double *x, int64_t ldx, int64_t n, const double *y, int64_t ldy, int64_t m, double *K_out,
@@ -1580,10 +1569,10 @@ static int gram_general(lgp_stream_t stream, const lgp_factor_t *factors, int nf
     const int vec_ok = ((ldk & 1) == 0) && ((reinterpret_cast<uintptr_t>(K_out) & 15) == 0);
     cudaStream_t st = (cudaStream_t)stream;
     if (devpar) {
-        if (general_smem_attr(gram_iso_kernel<true>, smem)) return LGP_ERR_CUDA;
+        if (smem_opt_in(gram_iso_kernel<true>, smem)) return LGP_ERR_CUDA;
         gram_iso_kernel<true><<<grid, G_THREADS, smem, st>>>(d, x, ldx, n, y, ldy, m, K_out, ldk, vec_ok, devpar);
     } else {
-        if (general_smem_attr(gram_iso_kernel<false>, smem)) return LGP_ERR_CUDA;
+        if (smem_opt_in(gram_iso_kernel<false>, smem)) return LGP_ERR_CUDA;
         gram_iso_kernel<false><<<grid, G_THREADS, smem, st>>>(d, x, ldx, n, y, ldy, m, K_out, ldk, vec_ok, nullptr);
     }
     LGP_CUDA_CHECK_LAUNCH();
@@ -1604,11 +1593,11 @@ static int vjp_general(lgp_stream_t stream, const lgp_factor_t *factors, int nfa
     const int64_t nblk = symlower ? tm * (tm + 1) / 2 : tm * tn;
     if (nblk > 2147483647LL) return LGP_ERR_UNSUPPORTED;
     if (devpar) {
-        if (general_smem_attr(gram_iso_vjp_kernel<true>, smem)) return LGP_ERR_CUDA;
+        if (smem_opt_in(gram_iso_vjp_kernel<true>, smem)) return LGP_ERR_CUDA;
         gram_iso_vjp_kernel<true><<<(unsigned)nblk, G_THREADS, smem, st>>>(d, x, ldx, n, y, ldy, m, G, ldg, b, symlower,
                                                                            (int)tn, out, devpar);
     } else {
-        if (general_smem_attr(gram_iso_vjp_kernel<false>, smem)) return LGP_ERR_CUDA;
+        if (smem_opt_in(gram_iso_vjp_kernel<false>, smem)) return LGP_ERR_CUDA;
         gram_iso_vjp_kernel<false><<<(unsigned)nblk, G_THREADS, smem, st>>>(d, x, ldx, n, y, ldy, m, G, ldg, b, symlower,
                                                                             (int)tn, out, nullptr);
     }
@@ -1631,11 +1620,11 @@ static int jvp_general(lgp_stream_t stream, const lgp_factor_t *factors, int nfa
     if (grid.y > 65535) return LGP_ERR_UNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
     if (devpar) {
-        if (general_smem_attr(gram_iso_jvp_kernel<true>, smem)) return LGP_ERR_CUDA;
+        if (smem_opt_in(gram_iso_jvp_kernel<true>, smem)) return LGP_ERR_CUDA;
         gram_iso_jvp_kernel<true><<<grid, G_THREADS, smem, st>>>(d, tan, x, ldx, n, y, ldy, m, D_out, ldd, devpar,
                                                                  tangent_dev);
     } else {
-        if (general_smem_attr(gram_iso_jvp_kernel<false>, smem)) return LGP_ERR_CUDA;
+        if (smem_opt_in(gram_iso_jvp_kernel<false>, smem)) return LGP_ERR_CUDA;
         gram_iso_jvp_kernel<false><<<grid, G_THREADS, smem, st>>>(d, tan, x, ldx, n, y, ldy, m, D_out, ldd, nullptr,
                                                                   nullptr);
     }
@@ -1719,8 +1708,11 @@ int lgp_gram_iso_vjp(lgp_stream_t stream, const lgp_factor_t *factors, int nfact
             int64_t t = (n + FT - 1) / FT;
             int64_t nblk = t * (t + 1) / 2;
             if (nblk > 2147483647LL) return LGP_ERR_UNSUPPORTED;
-#define LGP_VJP_LAUNCH(KIND, P) \
-    gram_fast_vjp_kernel<KIND, P><<<(unsigned)nblk, G_THREADS, smem, st>>>(fd, x, ldx, n, G, ldg, b, tmp)
+#define LGP_VJP_LAUNCH(KIND, P)                                                                       \
+    do {                                                                                              \
+        if (smem_opt_in(gram_fast_vjp_kernel<KIND, P>, smem)) return LGP_ERR_CUDA;                     \
+        gram_fast_vjp_kernel<KIND, P><<<(unsigned)nblk, G_THREADS, smem, st>>>(fd, x, ldx, n, G, ldg, b, tmp); \
+    } while (0)
             if (fd.kind == LGP_K_EXPQUAD)
                 LGP_VJP_LAUNCH(LGP_K_EXPQUAD, 0);
             else if (fd.kind == LGP_K_MATERNP && fd.p == 0)

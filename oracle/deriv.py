@@ -10,7 +10,7 @@ log(scale) and Cauchy beta differentiate the four numbers once more.  Terms use 
 
 import numpy as np
 
-from . import gp as ogp
+from . import gp as ogp, iso
 
 
 def kvmodx2_hi_ex(ex, x, q):
@@ -104,9 +104,9 @@ def factor_hd(f, x, y, a, b):
         v = ogp.factor_value(f, x, y)
         vl = ogp.factor_dlogscale(f, x, y)
         vb = zero
-        if kind == 'cauchy' and f.get('alpha', 2) == 2:
+        if kind == 'cauchy':
             u = _u_and_diffs(f, x, y, dims)[0]
-            vb = coefs('cauchy', u, beta=f.get('beta', 2))[1][0]
+            vb = iso.cauchy_dbeta(u, f.get('alpha', 2), f.get('beta', 2))
         return (v, zero, zero, zero), (vl, zero, zero, zero), (vb, zero, zero, zero)
     u, D = _u_and_diffs(f, x, y, dims)
     sx, sy = _pair(f.get('scale'), 1.0)

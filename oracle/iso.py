@@ -68,7 +68,8 @@ def kvmodx2(nu, x2, norm_offset=0):
         normal = 2 / special.gamma(nu + norm_offset) * (x / 2) ** nu * special.kv(nu, x)
     atzero = 1 / np.prod(nu + np.arange(norm_offset))
     atzero = np.where(nu > 0, atzero, 1)
-    return np.where(x2, normal, atzero)
+    # for nu > 0 the limit at x -> 0; there x^nu K_nu(x) is 0 * inf in float64 below x ~ 1e-300^(1/nu)
+    return np.where((x2 != 0) & ((nu <= 0) | np.isfinite(normal)), normal, atzero)
 
 
 def maternp_core(r2, p):
@@ -122,5 +123,20 @@ def matern_dr2(r2, nu):
 
 
 def cauchy_dr2(r2, alpha=2, beta=2):
-    assert alpha == 2
-    return -1 / 2 * (1 + r2 / beta) ** (-beta / 2 - 1)
+    # d/dr2 (1 + t/beta)^(-beta/alpha), t = r2^(alpha/2): -(1/2) (1 + t/beta)^(-beta/alpha - 1) t / r2; 0 at r2 = 0 for
+    # alpha < 2 (where it diverges), as the kernels: it only enters multiplied by r2
+    if alpha == 2:
+        return -1 / 2 * (1 + r2 / beta) ** (-beta / 2 - 1)
+    r2 = np.asarray(r2, dtype=float)
+    pos = r2 > 0
+    rp = np.where(pos, r2, 1.0)
+    t = rp ** (alpha / 2)
+    return np.where(pos, -1 / 2 * (1 + t / beta) ** (-beta / alpha - 1) * t / rp, 0.0)
+
+
+def cauchy_dbeta(r2, alpha=2, beta=2):
+    """ d/dbeta (1 + t/beta)^(-beta/alpha), t = r2^(alpha/2).  The two terms cancel to O(t^2) at small t: the result
+    is accurate to rounding relative to their size, (1 + t/beta)^(-beta/alpha) t / (alpha beta), not elementwise """
+    t = np.where(alpha == 2, r2, r2 ** (alpha / 2))
+    base = 1 + t / beta
+    return base ** (-beta / alpha) * (-np.log1p(t / beta) / alpha + t / (alpha * beta * base))

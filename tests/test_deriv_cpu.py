@@ -10,7 +10,7 @@ import pytest
 
 import lsqfitgp_b200 as lgp
 from lsqfitgp_b200 import _lib
-from oracle import deriv as od
+from oracle import deriv as od, gp as ogp
 
 ROOT = pathlib.Path(__file__).resolve().parent.parent
 
@@ -80,8 +80,8 @@ def test_linop_diff_errors():
 sympy = pytest.importorskip('sympy')
 import mpmath  # noqa: E402
 
-X0, X1, Y0, Y1, S, BETA = sympy.symbols('x0 x1 y0 y1 s beta', real=True)
-XS, YS = (X0, X1), (Y0, Y1)
+X0, X1, X2, Y0, Y1, Y2, S, BETA = sympy.symbols('x0 x1 x2 y0 y1 y2 s beta', real=True)
+XS, YS = (X0, X1, X2), (Y0, Y1, Y2)
 
 
 def _kv_hi(z, p):
@@ -93,7 +93,7 @@ def _kv_hi(z, p):
 
 
 def _sym_factor(f, scale_sym):
-    dims = f.get('dims', [0, 1])
+    dims = f.get('dims', [0, 1, 2])
     sx, sy = (scale_sym, scale_sym) if not isinstance(f.get('scale'), tuple) else f['scale']
     if f.get('scale') is None:
         sx = sy = 1
@@ -115,7 +115,13 @@ def _sym_factor(f, scale_sym):
 
 
 def _sym_kernel(terms):
-    return sum(amp * sympy.Mul(*[_sym_factor(f, S) for f in fs]) for amp, fs in terms)
+    # exact amplitudes: a float amplitude is a 15-digit sympy Float, which caps the precision of the cancellations at
+    # coincident points (the Maternp offset 1e-30 makes them cancel to about 15 digits)
+    return sum(sympy.Rational(repr(amp)) * _sym_term(fs) for amp, fs in terms)
+
+
+def _sym_term(factors):
+    return sympy.Mul(*[_sym_factor(f, S) for f in factors])
 
 
 SVAL, BVAL = 1.7, 1.3
@@ -132,38 +138,63 @@ def _cases():
         'sum_const': [(1.0, [dict(kind='maternp', p=2, scale=SVAL)]), (0.3, [dict(kind='constant')])],
         'loc': [(1.0, [dict(kind='maternp', p=1, scale=SVAL, loc=0.4)])],
         'tuple_scale': [(1.0, [dict(kind='expquad', scale=(1.3, 0.9), loc=(0.2, -0.1))])],
+        # both factors depend on field 0: both mixed products of the product rule are non-zero for (0, 0)
+        'shared_field': [(0.8, [dict(kind='expquad', dims=[0, 1], scale=SVAL),
+                                dict(kind='cauchy', alpha=2, beta=BVAL, dims=[0, 2], scale=SVAL)])],
+        # the differentiated field 2 is the second slot of the factor
+        'dims02': [(1.3, [dict(kind='maternp', p=2, dims=[0, 2], scale=SVAL)])],
+        # the second term does not depend on field 0; its Cauchy factor does not depend on field 1 either but carries
+        # scale and beta
+        'indep_term': [(1.0, [dict(kind='maternp', p=1, dims=[0, 1], scale=SVAL)]),
+                       (0.4, [dict(kind='expquad', dims=[1], scale=SVAL),
+                              dict(kind='cauchy', alpha=2, beta=BVAL, dims=[2], scale=SVAL)])],
     }
+
+
+NEW_CASES = ('shared_field', 'dims02', 'indep_term')
 
 
 def _points():
     rng = np.random.default_rng(5)
-    x = rng.uniform(-1, 1, (2, 4))
-    y = np.concatenate([x[:, :2], rng.uniform(-1, 1, (2, 2))], axis=1)  # two exactly coincident pairs
+    x = rng.uniform(-1, 1, (3, 4))
+    y = np.concatenate([x[:, :2], rng.uniform(-1, 1, (3, 2))], axis=1)  # two exactly coincident pairs
     return x, y
 
 
 def _sym_eval(expr, x, y, subs_extra):
     mpmath.mp.dps = 110
-    fn = sympy.lambdify((X0, X1, Y0, Y1, S, BETA), expr, modules='mpmath')
+    fn = sympy.lambdify((*XS, *YS, S, BETA), expr, modules='mpmath')
     out = np.empty((x.shape[1], y.shape[1]))
     for i in range(x.shape[1]):
         for j in range(y.shape[1]):
-            out[i, j] = float(fn(*[mpmath.mpf(v) for v in (x[0, i], x[1, i], y[0, j], y[1, j])], mpmath.mpf(SVAL),
-                                 mpmath.mpf(BVAL)))
+            out[i, j] = float(fn(*[mpmath.mpf(v) for v in (*x[:, i], *y[:, j])], mpmath.mpf(SVAL), mpmath.mpf(BVAL)))
     return out
+
+
+def _sym_block(expr, a, b):
+    if a is not None:
+        expr = sympy.diff(expr, XS[a])
+    if b is not None:
+        expr = sympy.diff(expr, YS[b])
+    return expr
 
 
 @pytest.mark.parametrize('name', list(_cases()))
 @pytest.mark.parametrize('a, b', [(0, None), (None, 1), (0, 0), (0, 1)])
 def test_oracle_vs_sympy(name, a, b):
+    _check_oracle_vs_sympy(name, a, b)
+
+
+@pytest.mark.parametrize('name', NEW_CASES)
+@pytest.mark.parametrize('a, b', [(2, None), (None, 2), (2, 2), (1, 2)])
+def test_oracle_vs_sympy_field2(name, a, b):
+    _check_oracle_vs_sympy(name, a, b)
+
+
+def _check_oracle_vs_sympy(name, a, b):
     terms = _cases()[name]
     x, y = _points()
-    k = _sym_kernel(terms)
-    expr = k
-    if a is not None:
-        expr = sympy.diff(expr, XS[a])
-    if b is not None:
-        expr = sympy.diff(expr, YS[b])
+    expr = _sym_block(_sym_kernel(terms), a, b)
     ref = _sym_eval(expr, x, y, {})
     got = od.block(terms, x, y, a, b)
     assert np.all(np.isfinite(got))
@@ -175,9 +206,14 @@ def test_oracle_vs_sympy(name, a, b):
     dl = sum(v for key, v in ders.items() if key[0] == 'logscale' and terms[key[1]][1][key[2]].get('scale'))
     ref_l = _sym_eval(S * sympy.diff(expr, S), x, y, {})
     np.testing.assert_allclose(dl, ref_l, rtol=1e-12, atol=1e-12 * max(np.max(np.abs(ref_l)), 1e-300))
-    if name == 'cauchy':
+    if any(f['kind'] == 'cauchy' for _, fs in terms for f in fs):
         ref_b = _sym_eval(sympy.diff(expr, BETA), x, y, {})
-        np.testing.assert_allclose(ders['beta', 0, 0], ref_b, rtol=1e-12, atol=1e-12 * np.max(np.abs(ref_b)))
+        db = sum(v for key, v in ders.items() if key[0] == 'beta')
+        np.testing.assert_allclose(db, ref_b, rtol=1e-12, atol=1e-12 * max(np.max(np.abs(ref_b)), 1e-300))
+    if name in NEW_CASES:
+        for ti, (_, fs) in enumerate(terms):
+            ref_a = _sym_eval(_sym_block(_sym_term(fs), a, b), x, y, {})
+            np.testing.assert_allclose(ders['amp', ti], ref_a, rtol=1e-12, atol=1e-12 * max(np.max(np.abs(ref_a)), 1e-300))
 
 
 @pytest.mark.parametrize('kind, kw, anchor', [
@@ -189,6 +225,52 @@ def test_r0_anchors(kind, kw, anchor):
     x = np.array([[0.3, -0.2]])
     K = od.block([(1.0, [dict(kind=kind, scale=s, **kw)])], x, x, 0, 0)
     np.testing.assert_allclose(np.diag(K), anchor / s ** 2, rtol=1e-15)
+
+
+# ---- hyperparameter derivatives of the plain cores (oracle.gp.factor_dlogscale, oracle.deriv.block_derivs) vs mpmath
+
+def _mp_core(kind, r2, nu=None, alpha=None, beta=None):
+    if kind == 'matern':
+        if r2 == 0:
+            return mpmath.mpf(1)
+        x = mpmath.sqrt(2 * nu * r2)
+        return 2 / mpmath.gamma(nu) * (x / 2) ** nu * mpmath.besselk(nu, x)
+    return (1 + r2 ** (alpha / 2) / beta) ** (-beta / alpha)
+
+
+# squared distances (before the scale 1.7): 0, tiny, moderate and large
+_R2 = [0.0, 1e-300, 1e-200, 1e-30, 1e-12, 1e-6, 0.01, 0.3, 1.0, 2.5, 10.0, 60.0]
+
+
+@pytest.mark.parametrize('kind, kw', [('matern', dict(nu=0.3)), ('matern', dict(nu=1.3)), ('matern', dict(nu=4.2)),
+                                      ('cauchy', dict(alpha=1.3, beta=0.7)), ('cauchy', dict(alpha=0.5, beta=3.0)),
+                                      ('cauchy', dict(alpha=2, beta=1.3))])
+def test_dlogscale_and_dbeta_vs_mpmath(kind, kw):
+    """ d/d log(scale) of every core and d/d beta of Cauchy of any alpha, on plain (underived) blocks, against mpmath
+    differentiation to 40 digits (working precision 360 digits: 1 + t / beta and the Bessel series cancel the digits
+    of tiny t) """
+    s = 1.7
+    x = np.sqrt(np.array(_R2))[None, :]
+    y = np.zeros((1, 1))
+    f = dict(kind=kind, scale=s, **kw)
+    got_l = ogp.factor_dlogscale(f, x, y)[:, 0]
+    ders = od.block_derivs([(1.0, [f])], x, y)
+    np.testing.assert_array_equal(ders['logscale', 0, 0][:, 0], got_l)
+    mpmath.mp.dps = 360
+    mkw = {k: mpmath.mpf(v) for k, v in kw.items()}
+    for i, r2 in enumerate(_R2):
+        R = mpmath.mpf(r2) / mpmath.mpf(s) ** 2
+        ref = mpmath.diff(lambda ls: _mp_core(kind, R * mpmath.exp(-2 * ls), **mkw), 0) if r2 else 0
+        assert abs(got_l[i] - float(ref)) <= 1e-13 * max(abs(float(ref)), 1e-300) + 1e-300, (r2, got_l[i], ref)
+        if kind == 'cauchy':
+            kb = dict(mkw)
+            del kb['beta']
+            ref_b = mpmath.diff(lambda b: _mp_core(kind, R, beta=b, **kb), mkw['beta'])
+            got_b = ders['beta', 0, 0][i, 0]
+            # d/dbeta = c (t / (alpha beta B) - log(B) / alpha), B = 1 + t/beta: the two terms cancel to O(t^2)
+            t = float(R / mpmath.mpf(s) ** 2) ** (kw['alpha'] / 2)
+            size = t / (kw['alpha'] * kw['beta'])
+            assert abs(got_b - float(ref_b)) <= 1e-13 * (abs(float(ref_b)) + size) + 1e-300, (r2, got_b, ref_b)
 
 
 # ---- host build of csrc/deriv_core.cuh vs the oracle
