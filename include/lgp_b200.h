@@ -19,9 +19,8 @@
  *   - thread safety: entry points may be called concurrently from several host threads on different streams
  *
  * Environment switches, for kernel experiments only (the product path needs none): LGP_TRACE (per-panel timeline of the
- * factorisation, synchronises), LGP_PANEL_BLOCKS (panel width in 128-blocks, default 4), LGP_GRAM_V3=0 (symmetric Gram
- * through the version-2 kernel), LGP_LEAF=1 (unblocked register-resident 128x128 leaf instead of chol_leaf3.cuh),
- * LGP_TAIL_BLOCKS / LGP_FIRST_BLOCKS / LGP_CHAIN_BLOCKS (panel schedule), LGP_GEMM_SMALL=0 (no latency tiles).
+ * factorisation, synchronises), LGP_PANEL_BLOCKS (panel width in 128-blocks, default 4), LGP_TAIL_BLOCKS /
+ * LGP_FIRST_BLOCKS / LGP_CHAIN_BLOCKS (panel schedule).
  */
 #ifndef LGP_B200_H
 #define LGP_B200_H
@@ -319,14 +318,13 @@ int lgp_chol_get_factor(lgp_stream_t stream, const double *W, int64_t ldw, const
 int lgp_chol_inverse(lgp_stream_t stream, const double *W, int64_t ldw, const double *aux, int64_t n,
                      double *scratch, double *Kinv, int64_t ldk);
 
-/* lgp_chol_factor followed by lgp_chol_inverse in ONE call, overlapped: what a logML + gradient evaluation needs
+/* lgp_chol_factor followed by lgp_chol_inverse in ONE call: what a logML + gradient evaluation needs
  * (Chol.__init__ and the invL / invK of minus_log_normal_density, src/lsqfitgp/_linalg/_decomp.py:380-393,466-472).
  * The factorisation runs on `stream` (on return the factor, aux and info are complete in `stream` order, exactly as after
  * lgp_chol_factor); the inverse runs on `inv_stream` (Kinv is complete in `inv_stream` order: make consumers wait for
  * that stream).  The inverse starts behind the complete factor; while it runs on `inv_stream` the caller's latency-bound
- * triangular solves on `stream` overlap its GEMMs.  (Starting the inverse of the leading half behind the half-way panel
- * was built and measured twice without gain, DESIGN.md section 3: experiment switch LGP_EARLY_INVERSE=1.)
- * inv_stream == stream gives the plain sequential composition.  Arguments as in the two calls. */
+ * triangular solves on `stream` overlap its GEMMs.  inv_stream == stream gives the plain sequential composition.
+ * Arguments as in the two calls. */
 int lgp_chol_factor_inverse(lgp_stream_t stream, lgp_stream_t inv_stream, const double *K, int64_t ldk,
                             const double *addmat, int64_t ldadd, const double *adddiag, int64_t n, double epsrel,
                             double epsabs, double *W, int64_t ldw, double *aux, int32_t *info, double *scratch,

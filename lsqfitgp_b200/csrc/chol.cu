@@ -109,191 +109,7 @@ __global__ void __launch_bounds__(1024) chol_jitter_kernel(int n, int npad, doub
 }
 
 // ------------------------------------------------------------------------------------------------
-// 2. leaf: 128x128 Cholesky + inverse of the factor, one CTA, matrix held in registers
-// ------------------------------------------------------------------------------------------------
-// Combined storage M[r][c]: r >= c holds A/L[r][c]; r < c holds row c of X = L^-1 (X[c][r]).
-// Thread (lane, w) owns rows lane+32a (a<4) and columns w+16b (b<8).  At step k the 32 lanes of warp
-// k%16 own column k, so the pivot is broadcast with one shuffle and there is a single barrier per step.
-constexpr int LEAF_THREADS = 256;
-constexpr int LEAF_SMEM_BYTES = (NB * (NB + 1) + 2 * NB) * 8;
-
-__device__ __forceinline__ void leaf_bar_sync(int id) {
-    asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(LEAF_THREADS) : "memory");
-}
-__device__ __forceinline__ void leaf_bar_arrive(int id) {
-    asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(LEAF_THREADS) : "memory");
-}
-
-// Thread (lane, w), w < 8: rows r = lane + 32a (a < 4), columns c = w + 8b (b < 16): M[a][b].
-// Combined storage: r >= c holds A/L[r][c]; r < c holds X[c][r], X = L^-1 (rows of X stored as columns).
-// Rank-1 update of step k on column block B (all indices static so that M stays in registers):
-//   M[r][c] -= col[r]*col[c]  for r >= c (Cholesky part) or r <= k (inverse part).
-template <int B>
-__device__ __forceinline__ void leaf_update_column(double (&M)[4][16], const double (&cr)[4], const bool (&rle)[4],
-                                                   const bool (&lowd)[4], double cc) {
-#pragma unroll
-    for (int a = 0; a < 4; a++) {
-        if (B < 4 * a) {  // block entirely below the diagonal
-            M[a][B] -= cr[a] * cc;
-        } else if (B >= 4 * a + 4) {  // entirely above: inverse part only
-            if (rle[a]) M[a][B] -= cr[a] * cc;
-        } else {  // block crossing the diagonal
-            if (lowd[B - 4 * a] || rle[a]) M[a][B] -= cr[a] * cc;
-        }
-    }
-}
-
-// Factor column k1 (held in M[.][B1] by the 32 lanes of this warp) after applying step k to it, and publish
-// col[r] = L[r][k1] (r > k1), X[k1][r] (r < k1), 1/L[k1][k1] (r == k1).
-template <int B1>
-__device__ __forceinline__ void leaf_next_column(double (&M)[4][16], const double (&cr)[4], const bool (&rle)[4],
-                                                 const bool (&lowd)[4], const double *col, double *colnext, int k1,
-                                                 int lane, int w, double *dvec, int32_t *info, int j0) {
-    constexpr int A1 = B1 >> 2;
-    leaf_update_column<B1>(M, cr, rle, lowd, col[w + 8 * B1]);
-    double pv = __shfl_sync(0xffffffffu, M[A1][B1], k1 & 31);
-    const double rl = rsqrt(pv);  // NaN for pv < 0, inf for pv == 0: propagates like a failed LAPACK/JAX factorisation
-    const double l = pv * rl;
-    if (lane == 0) {
-        if (!(pv > 0.0) || !(l < INFINITY)) atomicMin(info, j0 + k1 + 1);
-        dvec[j0 + k1] = l;
-    }
-#pragma unroll
-    for (int a = 0; a < 4; a++) {
-        const int r = lane + 32 * a;
-        const double v = M[a][B1] * rl;
-        colnext[r] = (r == k1) ? rl : v;
-        M[a][B1] = (r == k1) ? l : v;
-    }
-}
-
-template <int B, int BEND>
-struct LeafCols {
-    static __device__ __forceinline__ void run(double (&M)[4][16], const double (&cr)[4], const bool (&rle)[4],
-                                               const bool (&lowd)[4], const double *col, int w) {
-        if constexpr (B < BEND) {
-            leaf_update_column<B>(M, cr, rle, lowd, col[w + 8 * B]);
-            LeafCols<B + 1, BEND>::run(M, cr, rle, lowd, col, w);
-        }
-    }
-};
-
-// Steps k = 8*KB .. 8*KB+7 (columns of block KB; their owners are warps 0..7 in turn).
-template <int KB>
-__device__ __forceinline__ void leaf_block_steps(double (&M)[4][16], double *colbuf, int lane, int w,
-                                                 const bool (&lowd)[4], double *dvec, int32_t *info, int j0) {
-#pragma unroll 1
-    for (int kw = 0; kw < 8; kw++) {
-        const int k = 8 * KB + kw;
-        const double *col = colbuf + (k & 1) * NB;
-        double cr[4];
-        bool rle[4];
-#pragma unroll
-        for (int a = 0; a < 4; a++) {
-            cr[a] = col[lane + 32 * a];
-            rle[a] = (lane + 32 * a) <= k;
-        }
-        const int k1 = k + 1;
-        const bool next_owner = (k1 < NB) && (w == (k1 & 7));
-        // the warp owning column k+1 updates it first, factors it and releases the others (bar.arrive)
-        if (next_owner) {
-            double *colnext = colbuf + (k1 & 1) * NB;
-            if (kw < 7) {
-                leaf_next_column<KB>(M, cr, rle, lowd, col, colnext, k1, lane, w, dvec, info, j0);
-            } else {
-                if constexpr (KB + 1 < 16)
-                    leaf_next_column<KB + 1>(M, cr, rle, lowd, col, colnext, k1, lane, w, dvec, info, j0);
-            }
-            __threadfence_block();
-            leaf_bar_arrive(1 + (k1 & 1));
-        }
-        // column block KB: only columns c = w + 8*KB > k are still active
-        if ((w > kw) && !(next_owner && kw < 7)) leaf_update_column<KB>(M, cr, rle, lowd, col[w + 8 * KB]);
-        if constexpr (KB + 1 < 16) {
-            if (!(next_owner && kw == 7)) leaf_update_column<KB + 1>(M, cr, rle, lowd, col[w + 8 * (KB + 1)]);
-        }
-        LeafCols<KB + 2, 16>::run(M, cr, rle, lowd, col, w);
-        if (k1 < NB) {
-            if (next_owner)
-                __syncwarp();
-            else
-                leaf_bar_sync(1 + (k1 & 1));
-        }
-    }
-}
-
-template <int KB>
-struct LeafBlocks {
-    static __device__ __forceinline__ void run(double (&M)[4][16], double *colbuf, int lane, int w,
-                                               const bool (&lowd)[4], double *dvec, int32_t *info, int j0) {
-        if constexpr (KB < 16) {
-            leaf_block_steps<KB>(M, colbuf, lane, w, lowd, dvec, info, j0);
-            LeafBlocks<KB + 1>::run(M, colbuf, lane, w, lowd, dvec, info, j0);
-        }
-    }
-};
-
-__global__ void __launch_bounds__(LEAF_THREADS, 1) potrf_leaf_kernel(double *__restrict__ Wblk, int64_t ld,
-                                                                     double *__restrict__ invd,
-                                                                     double *__restrict__ dvec,
-                                                                     int32_t *__restrict__ info, int j0) {
-    extern __shared__ __align__(16) double leaf_sm[];
-    double *stage = leaf_sm;
-    double *colbuf = leaf_sm + NB * (NB + 1);
-    const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
-
-    for (int idx = tid; idx < NB * NB; idx += LEAF_THREADS) {
-        int r = idx >> 7, c = idx & 127;
-        stage[r * (NB + 1) + c] = Wblk[(int64_t)r * ld + c];
-    }
-    __syncthreads();
-    double M[4][16];
-#pragma unroll
-    for (int a = 0; a < 4; a++)
-#pragma unroll
-        for (int b = 0; b < 16; b++) {
-            int r = lane + 32 * a, c = w + 8 * b;
-            M[a][b] = (r >= c) ? stage[r * (NB + 1) + c] : 0.0;
-        }
-    bool lowd[4];
-#pragma unroll
-    for (int j = 0; j < 4; j++) lowd[j] = lane >= w + 8 * j;
-    // column 0 is factored by its owner (warp 0) before the loop
-    if (w == 0) {
-        double pv = __shfl_sync(0xffffffffu, M[0][0], 0);
-        const double rl = rsqrt(pv);
-        const double l = pv * rl;
-        if (lane == 0) {
-            if (!(pv > 0.0) || !(l < INFINITY)) atomicMin(info, j0 + 1);
-            dvec[j0] = l;
-        }
-#pragma unroll
-        for (int a = 0; a < 4; a++) {
-            const int r = lane + 32 * a;
-            const double v = M[a][0] * rl;
-            colbuf[r] = (r == 0) ? rl : v;
-            M[a][0] = (r == 0) ? l : v;
-        }
-    }
-    __syncthreads();
-    LeafBlocks<0>::run(M, colbuf, lane, w, lowd, dvec, info, j0);
-    __syncthreads();
-#pragma unroll
-    for (int a = 0; a < 4; a++)
-#pragma unroll
-        for (int b = 0; b < 16; b++) stage[(lane + 32 * a) * (NB + 1) + (w + 8 * b)] = M[a][b];
-    __syncthreads();
-    for (int idx = tid; idx < NB * NB; idx += LEAF_THREADS) {
-        int r = idx >> 7, c = idx & 127;
-        double lv = (r >= c) ? stage[r * (NB + 1) + c] : 0.0;
-        Wblk[(int64_t)r * ld + c] = lv;
-        double xv = (r > c) ? stage[c * (NB + 1) + r] : ((r == c) ? 1.0 / stage[r * (NB + 1) + r] : 0.0);
-        invd[idx] = xv;
-    }
-}
-
-// ------------------------------------------------------------------------------------------------
-// 3. small elementwise / reduction kernels
+// 2. small elementwise / reduction kernels
 // ------------------------------------------------------------------------------------------------
 constexpr int GRID_Y_MAX = 65535;
 // grid covering `cols` columns (256 per CTA) x `rows` rows, rows folded over (y, z) to respect the gridDim.y limit
@@ -370,29 +186,17 @@ __global__ void finalize_info_kernel(int32_t *info, int n) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// 4. host-side recursion (all sizes in 128-blocks of the padded matrix)
+// 3. host-side recursion (all sizes in 128-blocks of the padded matrix)
 // ------------------------------------------------------------------------------------------------
-// Leaf selection: version 3 (chol_leaf3.cuh) is the product path; version 1 (unblocked, register-resident; above) stays
-// selectable with LGP_LEAF=1 for A/B measurements.
-static int leaf_version() {
-    static const int v = [] {
-        const char *e = getenv("LGP_LEAF");
-        return (e && e[0] == '1') ? 1 : 3;
-    }();
-    return v;
-}
-static cudaError_t leaf_set_attrs() {
-    cudaError_t e = cudaFuncSetAttribute(potrf_leaf_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, LEAF_SMEM_BYTES);
-    if (e != cudaSuccess) return e;
-    return cudaFuncSetAttribute(potrf_leaf3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, L3_SMEM_BYTES);
-}
 // the > 48 KB shared-memory opt-in is a per-device attribute: once per device, not once per process
 static int leaf_attr() {
     static DeviceOnce once;
     const int dev = current_device();
     if (dev < 0) return LGP_ERR_CUDA;
     if (!once.done(dev)) {
-        if (leaf_set_attrs() != cudaSuccess) return LGP_ERR_CUDA;
+        if (cudaFuncSetAttribute(potrf_leaf3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, L3_SMEM_BYTES) !=
+            cudaSuccess)
+            return LGP_ERR_CUDA;
         once.set(dev);
     }
     return LGP_OK;
@@ -409,12 +213,8 @@ static int panel_blocks() {
     }();
     return v;
 }
-static void leaf_launch(cudaStream_t st, double *Wblk, int64_t ld, double *invd, double *dvec, int32_t *info, int j0,
-                        int version = 0) {
-    if ((version ? version : leaf_version()) == 3)
-        potrf_leaf3_kernel<<<1, L3_THREADS, L3_SMEM_BYTES, st>>>(Wblk, ld, invd, dvec, info, j0);
-    else
-        potrf_leaf_kernel<<<1, LEAF_THREADS, LEAF_SMEM_BYTES, st>>>(Wblk, ld, invd, dvec, info, j0);
+static void leaf_launch(cudaStream_t st, double *Wblk, int64_t ld, double *invd, double *dvec, int32_t *info, int j0) {
+    potrf_leaf3_kernel<<<1, L3_THREADS, L3_SMEM_BYTES, st>>>(Wblk, ld, invd, dvec, info, j0);
 }
 
 struct CholCtx {
@@ -536,17 +336,6 @@ static cudaStream_t panel_stream(cudaStream_t caller) {
 static inline bool ev_record(cudaEvent_t e, cudaStream_t s) { return e && cudaEventRecord(e, s) == cudaSuccess; }
 static inline bool ev_wait(cudaStream_t s, cudaEvent_t e) { return e && cudaStreamWaitEvent(s, e, 0) == cudaSuccess; }
 
-// Optional hook of the factorisation loop: called once, on the host, right after the panel that makes the leading
-// `blocks` block columns of the factor final (all rows) has been enqueued; `panel_done` is the event recorded behind that
-// panel on the panel stream.  lgp_chol_factor_inverse uses it to start the inverse of the leading half while the
-// factorisation's tail (bound by the panel chain, SMs mostly idle) is still running.
-struct PanelHook {
-    int blocks;
-    void (*fn)(void *ctx, cudaEvent_t panel_done);
-    void *ctx;
-    bool fired;
-};
-
 // Panel width (in 128-blocks) for a trailing matrix of `left` blocks.  Wide panels make the trailing rank-k updates
 // efficient while they dominate; once the trailing matrix is small the factorisation is bound by the chain of dependent
 // panel kernels, whose length per 128 columns grows with the recursion depth of the panel (4-block panel: 4 leaves + 17
@@ -590,7 +379,7 @@ static int first_blocks() {
     return v;
 }
 
-static int potrf_lookahead(CholCtx &cm, int nblk, int pb, PanelHook *hook = nullptr) {
+static int potrf_lookahead(CholCtx &cm, int nblk, int pb) {
     cudaStream_t ps = (nblk > pb) ? panel_stream(cm.st) : nullptr;
     if (!ps) {
         potrf_rec(cm, 0, nblk);
@@ -634,10 +423,6 @@ static int potrf_lookahead(CholCtx &cm, int nblk, int pb, PanelHook *hook = null
         e_last = e_panel;
         last = j;
         if ((rc = cp.rc) != LGP_OK || rest == 0 || !ok) break;
-        if (hook && !hook->fired && jb + w >= hook->blocks) {
-            hook->fired = true;
-            hook->fn(hook->ctx, e_panel);
-        }
         const int w2 = panel_width(rest, pb);  // width of the next panel
         const int rest2 = rest - w2;
         const int K = w * NB;
@@ -1207,10 +992,9 @@ int lgp_chol_factor_prepared(lgp_stream_t stream, int64_t n, double epsrel, doub
 }
 
 // debug/benchmark hook (not in the public header): run the 128x128 leaf `reps` times back to back
-int lgp_debug_leaf(lgp_stream_t stream, double *Wblk, int64_t ld, double *invd, double *dvec, int32_t *info, int reps,
-                   int variant) {
+int lgp_debug_leaf(lgp_stream_t stream, double *Wblk, int64_t ld, double *invd, double *dvec, int32_t *info, int reps) {
     if (leaf_attr()) return LGP_ERR_CUDA;
-    for (int i = 0; i < reps; i++) leaf_launch((cudaStream_t)stream, Wblk, ld, invd, dvec, info, 0, variant);
+    for (int i = 0; i < reps; i++) leaf_launch((cudaStream_t)stream, Wblk, ld, invd, dvec, info, 0);
     LGP_CUDA_CHECK_LAUNCH();
     return LGP_OK;
 }
@@ -1278,14 +1062,9 @@ int lgp_chol_get_factor(lgp_stream_t stream, const double *W, int64_t ldw, const
     return LGP_OK;
 }
 
-int lgp_chol_inverse(lgp_stream_t stream, const double *W, int64_t ldw, const double *aux, int64_t n64,
-                     double *scratch, double *Kinv, int64_t ldk) {
-    if (n64 < 1 || !W || !aux || !scratch || !Kinv) return LGP_ERR_BADARG;
-    const int n = (int)n64, npad = (int)lgp_chol_npad(n);
-    if (ldk < npad) return LGP_ERR_BADARG;
-    if ((ldk & 1) || (reinterpret_cast<uintptr_t>(Kinv) & 15) || (reinterpret_cast<uintptr_t>(scratch) & 15))
-        return LGP_ERR_ALIGN;
-    cudaStream_t st = (cudaStream_t)stream;
+// X = Lt^-1 into scratch (TRTRI), then Kinv = X^T X with the equilibration undone (LAUUM), on `st`
+static int chol_inverse_impl(cudaStream_t st, const double *W, int64_t ldw, const double *aux, int npad, double *scratch,
+                             double *Kinv, int64_t ldk) {
     InvCtx c{st, W, ldw, aux + LGP_AUX_INVDIAG(npad), scratch, (int64_t)npad, LGP_OK};
     const bool trace = trace_enabled();
     cudaEvent_t t0, t1, t2;
@@ -1313,115 +1092,35 @@ int lgp_chol_inverse(lgp_stream_t stream, const double *W, int64_t ldw, const do
     return LGP_OK;
 }
 
-// ---- factorisation and inverse-from-factor in one call, overlapped
-namespace lgp {
-struct EarlyInv {
-    InvCtx c;      // on the inverse stream
-    int nb, n1;    // blocks of the padded matrix, blocks of the leading half
-    bool ok;
-};
-// X11 = Lt11^-1 and Tt = X11^T L21^T: everything of the inverse that only needs the leading n1 block columns of the factor
-static void inverse_early(EarlyInv &e) {
-    InvCtx &c = e.c;
-    const int n1 = e.n1, n2 = e.nb - e.n1;
-    trtri_rec(c, 0, n1, 1, 2);
-    if (c.rc) return;
-    const double *L21 = c.W + (int64_t)n1 * NB * c.ldw;
-    double *Tt = c.X + (int64_t)n1 * NB;  // n1 x n2 scratch (upper block)
-    RC(gemm_launch(c.st, false, true, n1 * NB, n2 * NB, n1 * NB, 1.0, c.X, c.ldx, L21, c.ldw, Tt, c.ldx,
-                   GEMM_BETA0 | GEMM_A_UPPER_K));
+int lgp_chol_inverse(lgp_stream_t stream, const double *W, int64_t ldw, const double *aux, int64_t n64,
+                     double *scratch, double *Kinv, int64_t ldk) {
+    if (n64 < 1 || !W || !aux || !scratch || !Kinv) return LGP_ERR_BADARG;
+    const int n = (int)n64, npad = (int)lgp_chol_npad(n);
+    if (ldk < npad) return LGP_ERR_BADARG;
+    if ((ldk & 1) || (reinterpret_cast<uintptr_t>(Kinv) & 15) || (reinterpret_cast<uintptr_t>(scratch) & 15))
+        return LGP_ERR_ALIGN;
+    return chol_inverse_impl((cudaStream_t)stream, W, ldw, aux, npad, scratch, Kinv, ldk);
 }
-static void inverse_early_hook(void *ctx, cudaEvent_t panel_done) {
-    EarlyInv &e = *static_cast<EarlyInv *>(ctx);
-    if (!ev_wait(e.c.st, panel_done)) {
-        e.ok = false;  // could not order the inverse stream behind the panel: the early part runs later instead
-        return;
-    }
-    inverse_early(e);
-    e.ok = true;
-}
-}  // namespace lgp
 
+// ---- factorisation and inverse-from-factor in one call: the inverse runs on `inv_stream` behind the complete factor
 static int chol_factor_inverse_impl(lgp_stream_t stream, lgp_stream_t inv_stream, bool prepared, const double *K,
                                     int64_t ldk, const double *addmat, int64_t ldadd, const double *adddiag, int64_t n64,
                                     double epsrel, double epsabs, double *W, int64_t ldw, double *aux, int32_t *info,
                                     double *scratch, double *Kinv, int64_t ldkinv) {
-    if (n64 < 1 || n64 > (1 << 30) || (!prepared && !K) || !W || !aux || !info || !scratch || !Kinv) return LGP_ERR_BADARG;
-    const int n = (int)n64, npad = (int)lgp_chol_npad(n);
-    if (ldw < npad || (!prepared && (ldk < n || (addmat && ldadd < n))) || ldkinv < npad) return LGP_ERR_BADARG;
-    if ((ldw & 1) || (ldkinv & 1) || (reinterpret_cast<uintptr_t>(W) & 15) || (reinterpret_cast<uintptr_t>(aux) & 15) ||
-        (reinterpret_cast<uintptr_t>(Kinv) & 15) || (reinterpret_cast<uintptr_t>(scratch) & 15))
+    const int64_t npad = lgp_chol_npad(n64);
+    if (!scratch || !Kinv || ldkinv < npad) return LGP_ERR_BADARG;
+    if ((ldkinv & 1) || (reinterpret_cast<uintptr_t>(Kinv) & 15) || (reinterpret_cast<uintptr_t>(scratch) & 15))
         return LGP_ERR_ALIGN;
+    int rc = chol_factor_impl(stream, prepared, K, ldk, addmat, ldadd, adddiag, n64, epsrel, epsabs, W, ldw, aux, info);
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream, si = (cudaStream_t)inv_stream;
-    if (leaf_attr()) return LGP_ERR_CUDA;
-    if (epsrel < 0) epsrel = (double)n * 2.220446049250313e-16;
-    // the inverse stream starts behind whatever the caller has enqueued on the main stream (buffer reuse)
     if (si != st) {
-        cudaEvent_t e0 = ring_event();
-        if (!(ev_record(e0, st) && ev_wait(si, e0))) return LGP_ERR_CUDA;
-    }
-    if (!prepared) {
-        chol_diag_scale_kernel<<<(npad + 255) / 256, 256, 0, st>>>(K, ldk, addmat, ldadd, adddiag, n, npad, aux);
-        LGP_CUDA_CHECK_LAUNCH();
-        chol_prepare_kernel<<<(npad + 7) / 8, 256, 0, st>>>(K, ldk, addmat, ldadd, adddiag, n, npad, W, ldw, aux);
-        LGP_CUDA_CHECK_LAUNCH();
-    }
-    chol_jitter_kernel<<<1, 1024, 0, st>>>(n, npad, epsrel, epsabs, W, ldw, aux, info);
-    LGP_CUDA_CHECK_LAUNCH();
-    CholCtx c{st, W, ldw, aux + LGP_AUX_INVDIAG(npad), aux + LGP_AUX_DIAG(npad), info, LGP_OK};
-    const int nb = npad / NB;
-    EarlyInv early{InvCtx{si, W, ldw, aux + LGP_AUX_INVDIAG(npad), scratch, (int64_t)npad, LGP_OK}, nb, nb / 2, false};
-    PanelHook hook{early.n1, inverse_early_hook, &early, false};
-    // Early start of the inverse behind the half-way panel: OFF by default.  Measured on B200 at n = 20000 (round 2): the
-    // span of factorisation + inverse is unchanged (248.1 ms against 248.4 ms sequential) because the small, dependent
-    // kernels of the panel chain cannot get SM slots while long-K inverse GEMM CTAs saturate the GPU (the 128 x 128 leaf
-    // needs most of an SM's registers and shared memory, and freed single slots are back-filled by pending GEMM CTAs):
-    // the factorisation's tail stretches by exactly what the inverse gains.  Kept behind LGP_EARLY_INVERSE=1 for
-    // experiments; the call is otherwise the sequential composition on two streams.
-    static const bool early_on = [] {
-        const char *e = getenv("LGP_EARLY_INVERSE");
-        return e && e[0] == '1';
-    }();
-    const bool overlap = early_on && si != st && nb >= 8 * panel_blocks();
-    {
-        int rc = potrf_lookahead(c, nb, panel_blocks(), overlap ? &hook : nullptr);
-        if (rc) return rc;
-    }
-    finalize_info_kernel<<<1, 1, 0, st>>>(info, n);
-    LGP_CUDA_CHECK_LAUNCH();
-    logdet_quad_kernel<<<1, 1024, 0, st>>>(aux + LGP_AUX_DIAG(npad), aux + LGP_AUX_S(npad), nullptr, n,
-                                           aux + LGP_AUX_SCALARS(npad) + 4);
-    LGP_CUDA_CHECK_LAUNCH();
-    if (early.c.rc) return early.c.rc;
-    // ---- the rest of the inverse, behind the complete factor
-    if (si != st) {
-        cudaEvent_t e1 = ring_event();
-        if (!(ev_record(e1, st) && ev_wait(si, e1))) {
+        cudaEvent_t e = ring_event();
+        if (!(ev_record(e, st) && ev_wait(si, e))) {
             cudaStreamSynchronize(st);  // ordering could not be enqueued: fall back to a host-side join
         }
     }
-    InvCtx &ci = early.c;
-    if (nb == 1) {
-        trtri_rec(ci, 0, 1);
-    } else {
-        const int n1 = early.n1, n2 = nb - n1;
-        if (!(hook.fired && early.ok)) inverse_early(early);
-        if (ci.rc) return ci.rc;
-        trtri_rec(ci, n1, n2, 1, 3);
-        if (ci.rc) return ci.rc;
-        double *X22 = scratch + (int64_t)n1 * NB * npad + (int64_t)n1 * NB;
-        double *X21 = scratch + (int64_t)n1 * NB * npad;
-        double *Tt = scratch + (int64_t)n1 * NB;
-        // X21[i][j] = - sum_k X22[i][k] * Tt[j][k]  (k <= i)
-        int rc = gemm_launch(si, true, true, n2 * NB, n1 * NB, n2 * NB, -1.0, X22, npad, Tt, npad, X21, npad,
-                             GEMM_BETA0 | GEMM_A_LOWER_K);
-        if (rc) return rc;
-    }
-    if (ci.rc) return ci.rc;
-    int rc = gemm_launch(si, false, false, npad, npad, npad, 1.0, scratch, npad, scratch, npad, Kinv, ldkinv,
-                         GEMM_BETA0 | GEMM_LOWER | GEMM_A_UPPER_K, nullptr, aux + LGP_AUX_SINV(npad));
-    if (rc) return rc;
-    return LGP_OK;
+    return chol_inverse_impl(si, W, ldw, aux, (int)npad, scratch, Kinv, ldkinv);
 }
 
 int lgp_chol_factor_inverse(lgp_stream_t stream, lgp_stream_t inv_stream, const double *K, int64_t ldk,

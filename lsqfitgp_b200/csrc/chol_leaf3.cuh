@@ -1,6 +1,6 @@
 // 128x128 Cholesky leaf, version 3: Cholesky factor AND its inverse of one diagonal block in one CTA.
 //
-// Same contract as potrf_leaf_kernel (chol.cu): reads the lower triangle of Wblk, writes L into the lower triangle
+// Reads the lower triangle of Wblk, writes L into the lower triangle
 // (zeros above), X = L^-1 into invd (row-major 128 x 128, zeros above the diagonal), dvec[j0 + k] = L_kk, and
 // atomicMin(info, j0 + k + 1) at the first non-positive / non-finite pivot (NaNs then propagate like a failed
 // LAPACK/JAX factorisation, reference _linalg/_decomp.py:388-391).

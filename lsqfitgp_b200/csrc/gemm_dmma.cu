@@ -2,7 +2,6 @@
 #include "gemm_dmma.cuh"
 #include "internal.h"
 #include <math.h>
-#include <stdlib.h>
 #include <string.h>
 
 namespace lgp {
@@ -38,14 +37,6 @@ static int sm_count() {
         cached[dev] = v;
     }
     return cached[dev];
-}
-// experiment switch (read once): LGP_GEMM_SMALL=0 keeps the throughput tiles everywhere
-static bool gemm_small_disabled() {
-    static const bool v = [] {
-        const char *e = getenv("LGP_GEMM_SMALL");
-        return e && e[0] == '0';
-    }();
-    return v;
 }
 
 template <class Cfg>
@@ -85,7 +76,7 @@ int gemm_launch(cudaStream_t stream, bool a_kmaj, bool b_kmaj, int M, int N, int
     // idle with the throughput tiles use the latency tiles (4x the CTAs)
     const int sms = sm_count();
     if (flags & GEMM_INPLACE_B) {
-        const bool small = (N + 63) / 64 < sms && !gemm_small_disabled();
+        const bool small = (N + 63) / 64 < sms;
         if (a_kmaj && !b_kmaj)
             return small ? launch_cfg<GemmWideSmall, true, false>(stream, p) : launch_cfg<GemmWide, true, false>(stream, p);
         if (!a_kmaj && !b_kmaj)
@@ -94,14 +85,14 @@ int gemm_launch(cudaStream_t stream, bool a_kmaj, bool b_kmaj, int M, int N, int
         return LGP_ERR_UNSUPPORTED;
     }
     if (flags & GEMM_INPLACE_A) {
-        const bool small = (M + 63) / 64 < sms && !gemm_small_disabled();
+        const bool small = (M + 63) / 64 < sms;
         if (a_kmaj && b_kmaj)
             return small ? launch_cfg<GemmTallSmall, true, true>(stream, p) : launch_cfg<GemmTall, true, true>(stream, p);
         return LGP_ERR_UNSUPPORTED;
     }
     const int64_t tm = (M + 63) / 64, tn = (N + 63) / 64;
     const int64_t tiles = (flags & GEMM_LOWER) ? tm * (tm + 1) / 2 : tm * tn;
-    if (tiles < sms && !gemm_small_disabled()) return launch_layout<GemmSmall>(stream, a_kmaj, b_kmaj, p);
+    if (tiles < sms) return launch_layout<GemmSmall>(stream, a_kmaj, b_kmaj, p);
     return launch_layout<GemmBig>(stream, a_kmaj, b_kmaj, p);
 }
 

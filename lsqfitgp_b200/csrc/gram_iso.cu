@@ -801,11 +801,13 @@ struct GramPrep {
     double *rowpart;     // [npad / 64][npad]
     int64_t npad;
 };
-template <int KIND, int P, int MINB, bool PREP>
-__global__ void __launch_bounds__(G_THREADS, MINB) gram_fast3_kernel(const __grid_constant__ FastDesc d,
-                                                                  const double *__restrict__ x, int64_t ldx, int64_t n,
-                                                                  double *__restrict__ K, int64_t ldk, int vec_ok,
-                                                                  long long ntiles, const GramPrep prep) {
+// One lower tile per CTA, 3 CTAs per SM: at most 80 registers, and the launchers opt in to 77 400 bytes of shared memory
+// (3 * (76800 + 1024 reserved) = 228 KB)
+template <int KIND, int P, bool PREP>
+__global__ void __launch_bounds__(G_THREADS, 3) gram_fast3_kernel(const __grid_constant__ FastDesc d,
+                                                               const double *__restrict__ x, int64_t ldx, int64_t n,
+                                                               double *__restrict__ K, int64_t ldk, int vec_ok,
+                                                               const GramPrep prep) {
     extern __shared__ __align__(16) double fsm[];
     const int nd = d.nd;
     constexpr int F_TABREP = FTabRep<KIND>::value;
@@ -822,18 +824,12 @@ __global__ void __launch_bounds__(G_THREADS, MINB) gram_fast3_kernel(const __gri
     const int tid = threadIdx.x, ty = tid & 15, tx = tid >> 4;
     if (tid < 64 * F_TABREP) tab0[tid] = EXP_TAB_DEV[tid / F_TABREP];
     if (KIND == LGP_K_CAUCHY && tid < 64) reinterpret_cast<LogTab *>(fsm + 128 * F_TABREP)[tid] = LOG_TAB_DEV[tid];
-    // Persistent CTA: tiles b = blockIdx.x, blockIdx.x + gridDim.x, ...  The bulk stores of a tile are NOT waited for
-    // where they are issued: they drain while the points of the next tile are loaded and the first half of its entries
-    // is computed; the wait sits right before the staging buffers are written again.
-    bool pending = false;  // this thread has a committed bulk-store group that may still be reading D / T
-#pragma unroll 1
-    for (long long b = blockIdx.x; b < ntiles; b += gridDim.x) {
+    const long long b = blockIdx.x;  // lower tile b: row tm, column tn <= tm
     int tm = (int)((sqrtf(8.0f * (float)b + 1.0f) - 1.0f) * 0.5f);  // single precision + exact integer fix-up
     while ((long long)(tm + 1) * (tm + 2) / 2 <= b) tm++;
     while ((long long)tm * (tm + 1) / 2 > b) tm--;
     const int tn = (int)(b - (long long)tm * (tm + 1) / 2);
     const int64_t i0 = (int64_t)tm * FT, j0 = (int64_t)tn * FT;
-    __syncthreads();  // everybody is done with the staged points (and the non-bulk reads of T) of the previous tile
     for (int idx = tid; idx < nd * FT; idx += G_THREADS) {
         const int s = idx / FT, r = idx % FT;
         const int64_t i = i0 + r, j = j0 + r;
@@ -934,14 +930,6 @@ __global__ void __launch_bounds__(G_THREADS, MINB) gram_fast3_kernel(const __gri
                     }
             }
         }
-        if (a0 == 0) {
-            // D / T of the previous tile may still be read by its bulk stores: the issuing threads wait, then everybody
-            if (pending) {
-                asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-                pending = false;
-            }
-            __syncthreads();
-        }
         if (interior) {
 #pragma unroll
             for (int a = 0; a < 2; a++) {
@@ -998,7 +986,8 @@ __global__ void __launch_bounds__(G_THREADS, MINB) gram_fast3_kernel(const __gri
             asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(src), "r"(FT * 8)
                          : "memory");
             asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            pending = true;
+            // shared memory must stay valid until the bulk store has read it
+            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
         }
     } else if (mirror && !PREP) {
         __syncthreads();
@@ -1014,9 +1003,6 @@ __global__ void __launch_bounds__(G_THREADS, MINB) gram_fast3_kernel(const __gri
             }
         }
     }
-    }  // tile loop
-    // shared memory must stay valid until the last bulk stores have read it
-    if (pending) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
 }
 
 // d core / d r2 for the fast path (value returned through `val`)
@@ -1382,37 +1368,24 @@ static int launch_fast2(cudaStream_t st, const FastDesc &d, const double *x, int
     int64_t grid = sym ? tm * (tm + 1) / 2 : tm * tn;
     if (grid > 2147483647LL) return LGP_ERR_UNSUPPORTED;
     int vec_ok = ((ldk & 1) == 0) && ((reinterpret_cast<uintptr_t>(K) & 15) == 0);
-    static const bool v3 = !(getenv("LGP_GRAM_V3") && getenv("LGP_GRAM_V3")[0] == '0');  // A/B switch (experiments only)
     // version 3 stages both the tile and its mirror image and no raw coordinates; it needs 3 CTAs per SM to pay off
     const size_t smem3 = smem + (size_t)FT * F2_TS * 8 -
                          ((d.white_raw && FTabRep<KIND>::value != 1) ? (size_t)2 * d.nd * FT * sizeof(double) : 0);
-    if (sym && v3 && smem3 <= 77400) {
+    if (sym && smem3 <= 77400) {
         smem = smem3;
-        // 3 CTAs per SM (80 registers): measured 0.745 ms against 0.846 ms with 2 CTAs x 126 registers (Matern-5/2, n = 20k)
+        // 3 CTAs per SM (80 registers): measured 0.745 ms against 0.846 ms with 2 CTAs x 126 registers (Matern-5/2, n = 20k);
+        // many-field inputs that need more shared memory go through version 2
         static DeviceOnce once;
-        static int sm_count[MAX_DEVICES];
         const int dev = current_device();
         if (dev < 0) return LGP_ERR_CUDA;
         if (!once.done(dev)) {
-            if (cudaFuncSetAttribute(gram_fast3_kernel<KIND, P, 3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     77400) != cudaSuccess ||
-                cudaDeviceGetAttribute(&sm_count[dev], cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
+            if (cudaFuncSetAttribute(gram_fast3_kernel<KIND, P, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                     77400) != cudaSuccess)
                 return LGP_ERR_CUDA;
             once.set(dev);
         }
-        // (3 CTAs per SM: 3 * (76800 + 1024 reserved) = 228 KB; many-field inputs that need more go through version 2)
-        // one tile per CTA by default; LGP_GRAM_WAVES=k makes the CTAs persistent (k waves of 3 per SM walking the lower-tile
-        // list, bulk stores of a tile draining under the next tile's arithmetic): measured SLOWER on B200 at n = 20000
-        // (Matern-5/2: 0.805 ms with k = 1, 0.796 with k = 2, against 0.740 ms one tile per CTA: the hardware block scheduler
-        // balances the diagonal / edge tiles better than the static stride, and three resident CTAs already overlap the drain)
-        static const int waves = [] {  // A/B switch (experiments only): CTAs per SM-slot; 0 = one tile per CTA
-            const char *e = getenv("LGP_GRAM_WAVES");
-            return e ? atoi(e) : 0;
-        }();
-        const int64_t wave = waves > 0 ? (int64_t)3 * sm_count[dev] * waves : grid;
-        const unsigned g3 = (unsigned)(grid < wave ? grid : wave);
-        gram_fast3_kernel<KIND, P, 3, false><<<g3, G_THREADS, smem, st>>>(d, x, ldx, n, K, ldk, vec_ok, (long long)grid,
-                                                                          GramPrep{nullptr, nullptr, 0});
+        gram_fast3_kernel<KIND, P, false><<<(unsigned)grid, G_THREADS, smem, st>>>(d, x, ldx, n, K, ldk, vec_ok,
+                                                                                   GramPrep{nullptr, nullptr, 0});
     } else if (sym) {
         if (smem_opt_in(gram_fast2_kernel<KIND, P, true>, smem)) return LGP_ERR_CUDA;
         gram_fast2_kernel<KIND, P, true><<<(unsigned)grid, G_THREADS, smem, st>>>(d, x, ldx, n, y, ldy, m, K, ldk,
@@ -1491,7 +1464,7 @@ static int launch_prepare(cudaStream_t st, const FastDesc &d, const double *x, i
     const int dev = current_device();
     if (dev < 0) return LGP_ERR_CUDA;
     if (!once.done(dev)) {
-        if (cudaFuncSetAttribute(gram_fast3_kernel<KIND, P, 3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 77400) !=
+        if (cudaFuncSetAttribute(gram_fast3_kernel<KIND, P, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 77400) !=
             cudaSuccess)
             return LGP_ERR_CUDA;
         once.set(dev);
@@ -1500,8 +1473,8 @@ static int launch_prepare(cudaStream_t st, const FastDesc &d, const double *x, i
     if (grid > 2147483647LL) return LGP_ERR_UNSUPPORTED;
     gram_prep_diag_kernel<KIND><<<(unsigned)((npad + 255) / 256), 256, 0, st>>>(d, (int)n, (int)npad, aux);
     LGP_CUDA_CHECK_LAUNCH();
-    gram_fast3_kernel<KIND, P, 3, true><<<(unsigned)grid, G_THREADS, smem, st>>>(
-        d, x, ldx, n, W, ldw, 1, (long long)grid, GramPrep{aux + LGP_AUX_SINV(npad), work, npad});
+    gram_fast3_kernel<KIND, P, true><<<(unsigned)grid, G_THREADS, smem, st>>>(
+        d, x, ldx, n, W, ldw, 1, GramPrep{aux + LGP_AUX_SINV(npad), work, npad});
     LGP_CUDA_CHECK_LAUNCH();
     gram_prep_rowmax_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(work, npad, (int)t, (int)n, aux);
     LGP_CUDA_CHECK_LAUNCH();

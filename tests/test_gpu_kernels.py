@@ -527,8 +527,8 @@ def test_device_resident_descriptor_entry_points():
 
 @pytest.mark.parametrize('n', [300, 1500, 5000])
 def test_fused_factor_inverse_matches_separate_calls(n):
-    """ lgp_chol_factor_inverse (factorisation and inverse-from-factor overlapped on two streams, the leading half of the
-    inverse started behind the half-way panel for n >= 4096) gives the factor and inverse of the two separate calls """
+    """ lgp_chol_factor_inverse (factorisation on the main stream, inverse-from-factor on a second stream behind the
+    complete factor) gives the factor and inverse of the two separate calls """
     rng = np.random.default_rng(n)
     x = torch.tensor(rng.uniform(0, 10, (3, n)), device='cuda')
     descs = [dict(kind=_lib.K_MATERNP, term=0, dimmask=7, ipar=2, par0=0.0, scale_x=1.5, scale_y=1.5, amp=1.0),

@@ -1,5 +1,5 @@
 """Time the device part of one logML+gradient evaluation (Gram, factor + inverse on two streams, solves, Gram-VJP) at n:
-mean of `reps` after a warm-up; prints the separate phases as well.  Env switches (LGP_EARLY_INVERSE ...) are read once."""
+mean of `reps` after a warm-up; prints the separate phases as well.  Env switches (LGP_PANEL_BLOCKS ...) are read once."""
 import sys
 import numpy as np
 import torch
