@@ -194,7 +194,9 @@ int lgp_gram_bart(lgp_stream_t stream, int p, const int32_t *nsplits /*host*/, c
  *   for beta (each may be NULL; ld = ldd): what jax.jacfwd of the BART kernel gives `bayestree.bart`
  *   (src/lsqfitgp/bayestree/_bart.py:175-227 with forward=True, _fit.py:679-685).
  *   flags: LGP_BART_SYMMETRIC asserts ix == iy (same pointer) and n == m: only tiles on or below the diagonal are
- *   evaluated and mirrored. */
+ *   evaluated and mirrored.
+ *   More than LGP_BART_MAX_STAGES stages, LGP_BART_MAX_ROWS rows or 64 covariates of non-zero weight: LGP_ERR_UNSUPPORTED
+ *   (here and in lgp_gram_bart_vjp). */
 #define LGP_BART_MAX_ROWS 16
 #define LGP_BART_MAX_STAGES 8
 #define LGP_BART_SYMMETRIC 1

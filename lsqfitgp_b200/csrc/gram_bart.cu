@@ -354,8 +354,8 @@ static int bart_build(BartDesc &d, int p, const int32_t *nsplits, const double *
                       const int32_t *stage_nrows, const double *rows, const double *drows, double gamma, double amp,
                       int *need2, int *need3) {
     memset(&d, 0, sizeof(d));
-    if (p < 0 || (p && !nsplits) || nstages < 1 || nstages > B_MAX_STAGES || !stage_width || !stage_nrows || !rows)
-        return LGP_ERR_BADARG;
+    if (p < 0 || (p && !nsplits) || nstages < 1 || !stage_width || !stage_nrows || !rows) return LGP_ERR_BADARG;
+    if (nstages > B_MAX_STAGES) return LGP_ERR_UNSUPPORTED;
     int total = 0;
     *need2 = *need3 = 0;
     for (int s = 0; s < nstages; s++) {

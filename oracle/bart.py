@@ -51,9 +51,15 @@ def make_pnt(alpha, beta, maxd):
     return alpha / (1 + d) ** beta  # _bart.py:379-382
 
 
+def _inexact(x):
+    """ x as a float64 array, or complex128 when it is complex (the complex-step derivatives of gram_derivs) """
+    x = np.asarray(x)
+    return x.astype(np.result_type(x, float), copy=False)
+
+
 def fold_brackets(pnt, reset, altinput=True, debug=False):
     """ _bart.py:415-447 -> list of (probs, repeat) in evaluation order (deepest first) """
-    pnt = np.asarray(pnt, dtype=float)
+    pnt = _inexact(pnt)
     if reset is None:
         reset = []
     if not hasattr(reset, '__len__'):
@@ -95,12 +101,12 @@ def correlation(n, ix, iy, *, alpha=0.95, beta=2, gamma=1, maxd=2, debug=False, 
     if pnt is None:
         pnt = make_pnt(alpha, beta, maxd)
     else:
-        pnt = np.asarray(pnt, dtype=float)
+        pnt = _inexact(pnt)
     if weights is None:
-        weights = np.ones(n.shape[-1], pnt.dtype)
+        weights = np.ones(n.shape[-1])
     else:
         weights = np.asarray(weights, dtype=float)
-    gamma = np.asarray(gamma, dtype=float)
+    gamma = _inexact(gamma)
     if not intercept:
         pnt = pnt.copy()
         pnt[..., 0] = 1
@@ -118,9 +124,9 @@ def _correlation(n, ix, iy, pnt, gamma, w, debug=False, repeat=None, use_hash=Fa
     """ vectorised over leading axes of ix, iy and gamma; _bart.py:628-806 """
     n = np.asarray(n)
     ix, iy = np.broadcast_arrays(np.asarray(ix), np.asarray(iy))
-    pnt = np.asarray(pnt, dtype=float)
+    pnt = _inexact(pnt)
     w = np.asarray(w, dtype=float)
-    gamma = np.asarray(gamma, dtype=float)
+    gamma = _inexact(gamma)
     if repeat is not None:
         assert not debug and repeat > 0 and pnt.size % repeat == 0 and pnt.size // repeat <= 3
     else:
@@ -145,7 +151,7 @@ def _correlation(n, ix, iy, pnt, gamma, w, debug=False, repeat=None, use_hash=Fa
     if width == 1:
         for row in rows:
             gamma = np.where(anyn0, 1 - (1 - gamma) * row[0], 1)
-        return gamma + np.zeros(batch)
+        return gamma + np.zeros(batch, gamma.dtype)
 
     Wn = np.sum(np.where(n, w, 0))  # :694
 
@@ -319,8 +325,8 @@ def _correlation_old_vec(nminus, n0, nplus, pnt, gamma, w, debug):
     a = nminus.reshape(-1, nminus.shape[-1])
     b = n0.reshape(-1, n0.shape[-1])
     c = nplus.reshape(-1, nplus.shape[-1])
-    out = np.array([_correlation_old(a[q], b[q], c[q], np.asarray(pnt, float), float(g[q]), np.asarray(w, float),
-                                     debug) for q in range(a.shape[0])])
+    out = np.array([_correlation_old(a[q], b[q], c[q], _inexact(pnt), g[q], np.asarray(w, float), debug)
+                    for q in range(a.shape[0])])
     return out.reshape(batch)
 
 
@@ -328,7 +334,26 @@ def gram(n, ix, iy, *, chunk=256, **kw):
     """ full (len(ix), len(iy)) BART Gram matrix, row-chunked like batchufunc (_jaxext/_batcher.py:81-120) """
     ix = np.asarray(ix)
     iy = np.asarray(iy)
-    out = np.empty((ix.shape[0], iy.shape[0]))
+    cplx = any(np.iscomplexobj(kw.get(k)) for k in ('alpha', 'beta', 'gamma', 'pnt'))
+    out = np.empty((ix.shape[0], iy.shape[0]), complex if cplx else float)
     for s in range(0, ix.shape[0], chunk):
         out[s:s + chunk] = correlation(n, ix[s:s + chunk, None, :], iy[None, :, :], **kw)
     return out
+
+
+def _complex_step(f, n, ix, iy, alpha, beta, h, kw):
+    """ (f, df/dalpha, df/dbeta) with the derivatives Im f(alpha + ih) / h: alpha and beta enter only through
+    pnt_d = alpha / (1 + d)^beta, and everything after is +, -, *, / and index-selected branches, so there is no
+    subtractive cancellation and the result is exact to rounding """
+    return (f(n, ix, iy, alpha=alpha, beta=beta, **kw), f(n, ix, iy, alpha=alpha + 1j * h, beta=beta, **kw).imag / h,
+            f(n, ix, iy, alpha=alpha, beta=beta + 1j * h, **kw).imag / h)
+
+
+def correlation_derivs(n, ix, iy, *, alpha=0.95, beta=2, h=1e-200, **kw):
+    """ (correlation, d/dalpha, d/dbeta) per pair, by complex step """
+    return _complex_step(correlation, n, ix, iy, alpha, beta, h, kw)
+
+
+def gram_derivs(n, ix, iy, *, alpha=0.95, beta=2, h=1e-200, **kw):
+    """ (K, dK/dalpha, dK/dbeta) of `gram` (K without amplitude), by complex step """
+    return _complex_step(gram, n, ix, iy, alpha, beta, h, kw)

@@ -1,8 +1,9 @@
 """CPU accuracy test of the product's per-pair BART arithmetic (lsqfitgp_b200/csrc/bart_core.cuh, compiled for the host
 by oracle/Makefile into oracle/libbart_core_host.so) against the oracle restatement of the reference
 (oracle/bart.py <- src/lsqfitgp/_kernels/_bart.py:301-455,628-757): value (including the staged-reciprocal divisions and
-the index-selected digamma lookups), chained stages for reset patterns that do not fold into one bracket sequence, and
-the alpha / beta duals of the `repeat` scan against central finite differences of the oracle."""
+the index-selected digamma lookups), chained stages for reset patterns that do not fold into one bracket sequence, the
+alpha / beta duals of the `repeat` scan against the oracle's complex-step derivatives (exact to rounding), and the
+derivative rows `drows` of _BartSpec.stages() against the complex step of the bracket folding."""
 import ctypes
 import pathlib
 
@@ -101,22 +102,49 @@ def test_large_split_counts_value():
 
 
 @pytest.mark.parametrize('maxd,reset,intercept,weighted', CASES)
-def test_alpha_beta_duals_match_finite_differences(maxd, reset, intercept, weighted):
-    rng = np.random.default_rng(7 + maxd)
-    p = 5
-    nsplits, ix, iy = _problem(rng, p, 200, 30)
-    w = rng.uniform(0.2, 3, p) if weighted else np.ones(p)
-    alpha, beta, gamma = 0.9, 1.8, 0.6
-    spec = _BartSpec(1.0, (nsplits, None), True, alpha, beta, maxd, gamma, None, intercept, w, reset)
-    got = host_pairs(nsplits, w, spec, ix, iy)
-    h = 1e-5
+def test_alpha_beta_duals_match_complex_step(maxd, reset, intercept, weighted):
+    """ value and alpha / beta duals against the oracle's complex-step derivatives (exact to rounding), over covariate
+    counts, split counts from 3 to 4999 and (alpha, beta, gamma) including gamma = 0, alpha = 1 and beta = 0 """
+    for p in (1, 5, 9, 17):
+        for nmax in (3, 40, 4999):
+            rng = np.random.default_rng([maxd, p, nmax])
+            nsplits, ix, iy = _problem(rng, p, 200, nmax)
+            w = rng.uniform(0.2, 3, p) if weighted else np.ones(p)
+            if weighted and p > 2:
+                w[2] = 0.0      # a masked covariate
+            for alpha, beta, gamma in ((0.9, 1.8, 0.6), (1.0, 0.0, 1.0), (0.3, 4.0, 0.0)):
+                spec = _BartSpec(1.0, (nsplits, None), True, alpha, beta, maxd, gamma, None, intercept, w, reset)
+                got = host_pairs(nsplits, w, spec, ix, iy)
+                want = obart.correlation_derivs(nsplits, ix, iy, alpha=alpha, beta=beta, gamma=gamma, maxd=maxd,
+                                                intercept=intercept, weights=w, reset=reset)
+                what = (p, nmax, alpha, beta, gamma)
+                assert np.max(np.abs(got[:, 0] - want[0])) <= 1e-14, what
+                for k in (1, 2):
+                    ref = want[k]
+                    assert np.max(np.abs(got[:, k] - ref)) <= 2e-14 * np.max(np.abs(ref)), (what, k)
+                eq = np.all(np.where(w != 0, ix == iy, True), axis=1)
+                assert np.all(got[eq, 0] == 1) and np.all(got[eq, 1] == 0) and np.all(got[eq, 2] == 0), what
 
-    def corr(a, b):
-        return obart.correlation(nsplits, ix, iy, alpha=a, beta=b, gamma=gamma, maxd=maxd, intercept=intercept,
-                                 weights=w, reset=reset)
-    fa = (corr(alpha + h, beta) - corr(alpha - h, beta)) / (2 * h)
-    fb = (corr(alpha, beta + h) - corr(alpha, beta - h)) / (2 * h)
-    np.testing.assert_allclose(got[:, 1], fa, rtol=1e-7, atol=1e-9)
-    np.testing.assert_allclose(got[:, 2], fb, rtol=1e-7, atol=1e-9)
-    eq = np.all(np.where(w != 0, ix == iy, True), axis=1)
-    assert np.all(got[eq, 1] == 0) and np.all(got[eq, 2] == 0)
+
+@pytest.mark.parametrize('maxd,reset,intercept,weighted', CASES)
+def test_stage_drows_match_complex_step(maxd, reset, intercept, weighted):
+    """ _BartSpec.stages(): rows == the oracle's bracket folding, and drows == the complex step of make_pnt followed by
+    the folding; the entries the folding fixes to 1 (and pnt_0 without intercept) have derivative exactly 0 """
+    alpha, beta, h = 0.87, 1.9, 1e-200
+    spec = _BartSpec(1.0, (np.ones(3), None), True, alpha, beta, maxd, 0.5, None, intercept, None, reset)
+    widths, nrows, rows, drows, gamma = spec.stages()
+
+    def folded(a, b):
+        pnt = obart.make_pnt(a, b, maxd)
+        if not intercept:
+            pnt[0] = 1
+        out = []
+        for probs, repeat in obart.fold_brackets(pnt, reset):
+            r = probs.reshape(repeat or 1, -1)
+            out.append(np.concatenate([r, np.ones((len(r), 3 - r.shape[1]))], axis=1))
+        return np.concatenate(out)
+    assert np.array_equal(rows, folded(alpha, beta))
+    for k, ref in enumerate([folded(alpha + 1j * h, beta).imag / h, folded(alpha, beta + 1j * h).imag / h]):
+        np.testing.assert_allclose(drows[k], ref, rtol=1e-15, atol=0, err_msg=str(k))
+        assert np.all(drows[k][ref == 0] == 0)
+    assert np.all(drows[:, rows == 1] == 0)

@@ -1,7 +1,7 @@
 """GPU parity of the BART path added in round 2: chained bracket stages (reset patterns that do not fold into one
-`repeat` sequence, reference _kernels/_bart.py:447-455), symmetric evaluation, alpha / beta derivatives (forward
-matrices and the fused reverse contraction), gradients through the public API, and the `bayestree.bart` recipe
-(reference bayestree/_bart.py:147-240) fitted end to end against the oracle's objective."""
+`repeat` sequence, reference _kernels/_bart.py:447-455), symmetric evaluation, alpha / beta gradients through the
+public API in reverse and forward mode (the kernels themselves are checked in test_gpu_bart_exact.py), and the
+`bayestree.bart` recipe (reference bayestree/_bart.py:147-240) fitted end to end against the oracle's objective."""
 import numpy as np
 import pytest
 import torch
@@ -9,7 +9,6 @@ from scipy import optimize, stats
 
 import lsqfitgp_b200 as lgp
 from lsqfitgp_b200 import _ops
-from lsqfitgp_b200._kernels import _BartSpec
 from oracle import gp as ogp, bart as obart
 
 pytestmark = pytest.mark.gpu
@@ -52,68 +51,64 @@ def test_chained_stages_and_symmetry_vs_oracle(kw):
     assert torch.equal(Ks, Kg)
 
 
-@pytest.mark.parametrize('kw', [dict(maxd=10, reset=[2, 4, 6, 8]), dict(maxd=3, reset=[1]), dict(maxd=2), dict(maxd=1),
-                                dict(maxd=6, reset=[1, 2, 4], intercept=False, gamma=0.7)])
-def test_alpha_beta_derivatives_and_vjp(kw):
-    X, splits, idx = _data(210, seed=11)
-    alpha, beta = 0.9, 1.7
-    spec = _BartSpec(1.3, splits, True, alpha, beta, kw['maxd'], kw.get('gamma', 1), None, kw.get('intercept', True), None,
-                     kw.get('reset'))
-    widths, nrows, rows, drows, gamma = spec.stages()
-    w = np.ones(idx.shape[1])
-    ix = _dev_idx(idx)
-    iy = _dev_idx(idx[:150])
-    K, dKa, dKb = _ops.gram_bart_stages(splits[0], w, widths, nrows, rows, drows, gamma, 1.3, ix, iy, deriv=True)
-    okw = {k: v for k, v in kw.items()}
-    h = 1e-5
-
-    def corr(a, b):
-        return 1.3 * obart.gram(splits[0], idx, idx[:150], alpha=a, beta=b, **okw)
-    assert np.max(np.abs(K.cpu().numpy() - corr(alpha, beta)) / corr(alpha, beta)) < 1e-13
-    fa = (corr(alpha + h, beta) - corr(alpha - h, beta)) / (2 * h)
-    fb = (corr(alpha, beta + h) - corr(alpha, beta - h)) / (2 * h)
-    np.testing.assert_allclose(dKa.cpu().numpy(), fa, rtol=1e-6, atol=1e-8)
-    np.testing.assert_allclose(dKb.cpu().numpy(), fb, rtol=1e-6, atol=1e-8)
-    # reverse mode, dense cotangent: sum_ij G_ij {corr, dK/dalpha, dK/dbeta}
-    G = torch.randn(K.shape, dtype=torch.float64, device=DEV, generator=torch.Generator(DEV).manual_seed(3))
-    v = _ops.gram_bart_vjp(splits[0], w, widths, nrows, rows, drows, gamma, 1.3, ix, iy, _ops.as_aligned(G)).cpu().numpy()
-    want = np.array([float((G * K).sum()) / 1.3, float((G * dKa).sum()), float((G * dKb).sum())])
-    np.testing.assert_allclose(v, want, rtol=1e-11, atol=1e-11 * np.abs(want).max())
-    # symmetric form: lower triangle of a symmetric G, G_ij - b_i b_j, weights 2 off the diagonal
-    Ks, dKas, dKbs = _ops.gram_bart_stages(splits[0], w, widths, nrows, rows, drows, gamma, 1.3, ix, ix, deriv=True,
-                                           symmetric=True)
-    A = torch.randn((len(idx), len(idx)), dtype=torch.float64, device=DEV, generator=torch.Generator(DEV).manual_seed(4))
-    Gs = A + A.T
-    b = torch.randn(len(idx), dtype=torch.float64, device=DEV, generator=torch.Generator(DEV).manual_seed(5))
-    low = torch.tril(Gs) + torch.triu(torch.full_like(Gs, float('nan')), 1)   # the upper triangle must not be read
-    vs = _ops.gram_bart_vjp(splits[0], w, widths, nrows, rows, drows, gamma, 1.3, ix, ix, _ops.as_aligned(low), b=b,
-                            symlower=True).cpu().numpy()
-    Gf = Gs - torch.outer(b, b)
-    wants = np.array([float((Gf * Ks).sum()) / 1.3, float((Gf * dKas).sum()), float((Gf * dKbs).sum())])
-    np.testing.assert_allclose(vs, wants, rtol=1e-11, atol=1e-11 * np.abs(wants).max())
-
-
 def test_alpha_beta_gradient_through_api():
-    """ d logML / d (alpha, beta, amplitude) by torch.autograd through lgp_gram_bart_vjp against central differences of
-    the oracle's logML (the derivatives the reference gets by tracing _bart.py with JAX) """
-    X, splits, idx = _data(240, seed=21)
+    """ d logML / d (alpha, beta, amplitude) by torch.autograd through lgp_gram_bart_vjp against
+    -1/2 tr(K^-1 dK) + 1/2 b' dK b, b = K^-1 y, with dK from the oracle's complex-step derivatives (the derivatives the
+    reference gets by tracing _bart.py with JAX): one folded width-3 stage on 6 columns, and chained stages on 17
+    columns of which one has weight 0 """
+    w17 = np.r_[np.ones(9), 0.0, np.linspace(0.5, 2, 7)]
+    for p, kw in ((6, dict(maxd=10, reset=[2, 4, 6, 8])), (17, dict(maxd=6, reset=[1, 2, 4], weights=w17))):
+        X, splits, idx = _data(240, seed=21, p=p)
+        n = len(idx)
+        xi = lgp.unstructured_to_structured(idx.astype(np.int32), names=[f'c{i}' for i in range(idx.shape[1])])
+        y = np.random.default_rng(5).standard_normal(n)
+        t0 = np.array([0.9, 1.6, 1.2])
+        th = torch.tensor(t0, dtype=torch.float64, requires_grad=True)
+        kb = th[2] ** 2 * lgp.BART(splits=splits, indices=True, alpha=th[0], beta=th[1], **kw)
+        gp = (lgp.GP(kb, checkpos=False, checksym=False, epsrel=0).addx(xi, 'f').addcov(0.3 * np.eye(n), 'e')
+              .addtransf({'f': 1, 'e': 1}, 'y'))
+        ml = gp.marginal_likelihood({'y': y})
+        g, = torch.autograd.grad(ml, th)
+        Kb, dKa, dKb = obart.gram_derivs(splits[0], idx, idx, alpha=t0[0], beta=t0[1], **kw)
+        Ko = t0[2] ** 2 * Kb + 0.3 * np.eye(n)
+        assert abs(float(ml.detach()) - ogp.logml(Ko, y, epsrel=0)) <= 1e-9 * abs(ogp.logml(Ko, y, epsrel=0)), p
+        Ki = np.linalg.inv(Ko)
+        b = Ki @ y
+        want = np.array([-0.5 * np.sum(Ki * dK) + 0.5 * b @ dK @ b
+                         for dK in (t0[2] ** 2 * dKa, t0[2] ** 2 * dKb, 2 * t0[2] * Kb)])
+        assert np.max(np.abs(g.numpy() - want)) <= 1e-9 * np.max(np.abs(want)), (p, g.numpy(), want)
+
+
+def test_empbayes_fit_fisher_bart():
+    """ method='fisher' on a BART GP runs the BART forward mode (lgp_gram_bart_stages with derivatives, through the
+    Gram JVP of the public API): amplitude and noise fitted in log space, alpha = sigmoid(za) and beta = exp(zb) mapped
+    by torch ops.  minresult.hess - I equals the oracle's 1/2 tr(K^-1 dK_i K^-1 dK_j) (prior sdev 1: identity
+    jacobian), with dK/dp_i by complex step through the parameter maps and the BART correlation """
+    X, splits, idx = _data(200, seed=31)
     n = len(idx)
     xi = lgp.unstructured_to_structured(idx.astype(np.int32), names=[f'c{i}' for i in range(idx.shape[1])])
-    y = np.random.default_rng(5).standard_normal(n)
-    th = torch.tensor([0.9, 1.6, 1.2], dtype=torch.float64, requires_grad=True)
-    kb = th[2] ** 2 * lgp.BART(splits=splits, indices=True, alpha=th[0], beta=th[1], maxd=10, reset=[2, 4, 6, 8])
-    gp = (lgp.GP(kb, checkpos=False, checksym=False, epsrel=0).addx(xi, 'f').addcov(0.3 * np.eye(n), 'e')
-          .addtransf({'f': 1, 'e': 1}, 'y'))
-    ml = gp.marginal_likelihood({'y': y})
-    g, = torch.autograd.grad(ml, th)
+    rng = np.random.default_rng(32)
+    y = np.sin(X[:, 0]) + 0.5 * X[:, 4] + 0.3 * rng.standard_normal(n)
+    hyperprior = {'log(amp)': (0.0, 1.0), 'log(noise)': (np.log(0.3), 1.0), 'za': (1.0, 1.0), 'zb': (0.5, 1.0)}
+    bkw = dict(maxd=10, reset=[2, 4, 6, 8])
 
-    def f(t):
-        Ko = t[2] ** 2 * obart.gram(splits[0], idx, idx, alpha=t[0], beta=t[1], maxd=10, reset=[2, 4, 6, 8]) + 0.3 * np.eye(n)
-        return ogp.logml(Ko, y, epsrel=0)
-    t0 = th.detach().numpy()
-    assert abs(float(ml.detach()) - f(t0)) <= 1e-9 * abs(f(t0))
-    fd = np.array([(f(t0 + h) - f(t0 - h)) / 2e-5 for h in 1e-5 * np.eye(3)])
-    np.testing.assert_allclose(g.numpy(), fd, rtol=2e-6, atol=1e-7)
+    def gpfactory(hp):
+        k = hp['amp'] ** 2 * lgp.BART(splits=splits, indices=True, alpha=torch.sigmoid(hp['za']),
+                                      beta=torch.exp(hp['zb']), **bkw) + hp['noise'] ** 2 * lgp.White()
+        return lgp.GP(k, checkpos=False, checksym=False).addx(xi, 'data')
+    fit = lgp.empbayes_fit(hyperprior, gpfactory, {'data': y}, raises=False, method='fisher')
+    mean = np.array([v[0] for v in hyperprior.values()])
+
+    def Kof(pv):
+        la, ln, za, zb = mean + pv
+        Kb = obart.gram(splits[0], idx, idx, alpha=1 / (1 + np.exp(-za)), beta=np.exp(zb), **bkw)
+        return np.exp(2 * la) * Kb + np.exp(2 * ln) * np.eye(n)
+    x = fit.minresult.x
+    h = 1e-200
+    Ki = np.linalg.inv(Kof(x))
+    A = [Ki @ (Kof(x + 1j * h * e).imag / h) for e in np.eye(4)]
+    fo = np.array([[0.5 * np.sum(a * b.T) for b in A] for a in A])
+    assert np.max(np.abs(fit.minresult.hess - np.eye(4) - fo)) <= 1e-9 * np.max(np.abs(fo)), (fit.minresult.hess, fo)
 
 
 def test_bayestree_bart_fit_vs_oracle():

@@ -75,7 +75,9 @@ def test_structured_array():
                                         (3, [1]), (6, [1, 2, 4]), (7, [2, 3, 5])])
 def test_bart_bracket_folding_matches_oracle(maxd, reset):
     """ stages (including reset patterns that do not fold into one `repeat` sequence: chained stages) against the
-    oracle's restatement of the reference's bracket folding, and the derivative rows against finite differences """
+    oracle's restatement of the reference's bracket folding, and the derivative rows against the complex step of the
+    folding (exact to rounding; the same check as tests/test_bart_core_cpu.py::test_stage_drows_match_complex_step on
+    these reset patterns) """
     spec = _BartSpec(1.0, (np.array([3]), None), True, 0.95, 2, maxd, 1, None, True, None, reset)
     widths, nrows, rows, drows, gamma = spec.stages()
     ref = obart.fold_brackets(obart.make_pnt(0.95, 2, maxd), reset)
@@ -86,11 +88,13 @@ def test_bart_bracket_folding_matches_oracle(maxd, reset):
         np.testing.assert_array_equal(rows[r:r + nr, :w].ravel(), probs)
         r += nr
     assert r == len(rows) and drows.shape == (2,) + rows.shape
-    h = 1e-6
-    for q, (da, db) in enumerate([(h, 0.0), (0.0, h)]):
-        up = _BartSpec(1.0, (np.array([3]), None), True, 0.95 + da, 2 + db, maxd, 1, None, True, None, reset).stages()[2]
-        dn = _BartSpec(1.0, (np.array([3]), None), True, 0.95 - da, 2 - db, maxd, 1, None, True, None, reset).stages()[2]
-        np.testing.assert_allclose(drows[q], (up - dn) / (2 * h), atol=1e-8)
+    h = 1e-200
+    for q, (a, b) in enumerate([(0.95 + 1j * h, 2), (0.95, 2 + 1j * h)]):
+        r = 0
+        for w, nr, (probs, repeat) in zip(widths, nrows, obart.fold_brackets(obart.make_pnt(a, b, maxd), reset)):
+            np.testing.assert_allclose(drows[q, r:r + nr, :w], probs.imag.reshape(nr, w) / h, rtol=1e-15, atol=0)
+            assert np.all(drows[q, r:r + nr, w:] == 0)
+            r += nr
 
 
 def test_bart_unsupported_depth():

@@ -148,3 +148,49 @@ def test_c_restatement(rng):
         c_c = f(p, n.ctypes.data_as(i64p), ix.ctypes.data_as(i64p), iy.ctypes.data_as(i64p), w.ctypes.data_as(dp),
                 rows.ctypes.data_as(dp), repeat, 0.7)
         assert abs(c_np - c_c) <= 1e-14 * abs(c_np)
+
+
+def _cs(f, x, h=1e-200):
+    """ complex-step derivative Im f(x + ih) / h """
+    return np.imag(f(x + 1j * h)) / h
+
+
+@pytest.mark.parametrize('md,reset', [(1, None), (2, None), (3, [1]), (4, [2])])
+def test_complex_step_closed_forms_vs_old_recursion(md, reset, rng):
+    """ d/dalpha and d/dbeta by complex step through the closed forms (altinput) == the same through the independent
+    older implementation: the complex-step oracle of gram_derivs does not inherit an error of one formulation """
+    for _ in range(4):
+        p = int(rng.integers(1, 7))
+        n = rng.integers(0, 25, p)
+        ix, iy = rng.integers(0, n + 1, (2, 40, p))
+        iy[:5] = ix[:5]                     # coinciding points
+        w = rng.uniform(0.2, 3, p)
+        w[rng.random(p) < 0.25] = 0.0
+        nm, n0, npl = np.minimum(ix, iy), np.abs(ix - iy), n - np.maximum(ix, iy)
+        alpha, beta, gamma = rng.uniform(0.1, 1), rng.uniform(0, 4), rng.choice([0.0, 1.0, rng.uniform()])
+        kw = dict(gamma=gamma, maxd=md, reset=reset, weights=w)
+
+        def new(a, b):
+            return bart.correlation(n, ix, iy, alpha=a, beta=b, **kw)
+
+        def old(a, b):
+            return bart.correlation(nm, n0, npl, alpha=a, beta=b, altinput=False, **kw)
+        for d1, d2 in [(_cs(lambda a: new(a, beta), alpha), _cs(lambda a: old(a, beta), alpha)),
+                       (_cs(lambda b: new(alpha, b), beta), _cs(lambda b: old(alpha, b), beta))]:
+            assert np.max(np.abs(d1 - d2)) <= 1e-14 * np.max(np.abs(d2)), (np.max(np.abs(d1 - d2)), np.max(np.abs(d2)))
+            assert np.all(d1[:5] == 0)
+
+
+def test_gram_derivs_vs_central_differences(rng):
+    """ sanity of gram_derivs' complex step against central differences of the real oracle """
+    n = rng.integers(0, 30, 6)
+    ix, iy = rng.integers(0, n + 1, (2, 30, 6))
+    kw = dict(maxd=10, reset=[2, 4, 6, 8], gamma=0.6)
+    alpha, beta, h = 0.9, 1.7, 1e-5
+    K, dKa, dKb = bart.gram_derivs(n, ix, iy, alpha=alpha, beta=beta, **kw)
+    assert K.dtype == dKa.dtype == dKb.dtype == float
+    assert np.array_equal(K, bart.gram(n, ix, iy, alpha=alpha, beta=beta, **kw))
+    fa = (bart.gram(n, ix, iy, alpha=alpha + h, beta=beta, **kw) - bart.gram(n, ix, iy, alpha=alpha - h, beta=beta, **kw))
+    fb = (bart.gram(n, ix, iy, alpha=alpha, beta=beta + h, **kw) - bart.gram(n, ix, iy, alpha=alpha, beta=beta - h, **kw))
+    np.testing.assert_allclose(dKa, fa / (2 * h), rtol=1e-7, atol=1e-9)
+    np.testing.assert_allclose(dKb, fb / (2 * h), rtol=1e-7, atol=1e-9)
