@@ -123,6 +123,18 @@ int lgp_gram_iso_jvp(lgp_stream_t stream, const lgp_factor_t *factors, int nfact
                      int64_t ldx, int64_t n, const double *y, int64_t ldy, int64_t m, const double *tangent,
                      double *D_out, int64_t ldd);
 
+/* Second-order contraction of the Gram build, the derivative of lgp_gram_iso_vjp along `tangent` (what a second
+ * jax.vjp through the Gram build gives the reference's Hessian, src/lsqfitgp/_fit.py empbayes_fit(method='hessian'),
+ * without materialising the k^2 matrices d2K/dtheta_a dtheta_b):
+ *   out[3f+k] = sum_ij G_ij d/dtheta_{f,k} ( sum_{g,l} tangent[3g+l] dK_ij/dtheta_{g,l} ),
+ *   theta_{f,.} = (amp_f, log(scale_f), par1_f)      (scale_x == scale_y == scale_f)
+ * G, b and symlower as in lgp_gram_iso_vjp; `tangent` is HOST memory (3*nfactors doubles, the layout of
+ * lgp_gram_iso_jvp).  Every kind of the general kernel.  out: device memory, 3*nfactors doubles (zeroed by the call;
+ * accumulated with atomicAdd). */
+int lgp_gram_iso_hvp(lgp_stream_t stream, const lgp_factor_t *factors, int nfactors, int ndim, const double *x,
+                     int64_t ldx, int64_t n, const double *y, int64_t ldy, int64_t m, const double *G, int64_t ldg,
+                     const double *b, int symlower, const double *tangent, double *out);
+
 /* Derivative blocks: the covariance between first derivatives of the process, cov(d f(x)/d x_a, d f(y)/d y_b), with
  * a = dx_field, b = dy_field (field indices; -1 = no derivative on that argument, both -1 is LGP_ERR_BADARG).
  * Replaces the reference's jax derivatives of the kernel core behind addx(deriv=) and CrossKernel.linop('diff')

@@ -105,6 +105,13 @@ class _GramFn(torch.autograd.Function):
     def backward(ctx, G):
         kern, xd, yd, labels, dfields = ctx.kern, ctx.xd, ctx.yd, ctx.labels, ctx.dfields
         hyper = kern._hyperparams()
+        if torch.is_grad_enabled():   # create_graph: the gradient itself must be differentiable
+            why = _no_second_order(hyper, dfields)
+            if why is None:
+                return (None, None, None, None, None, *_gram_vjp_graph(kern, xd, yd, labels, G, hyper))
+            with torch.no_grad():
+                grads = _GramFn.backward(ctx, G.detach())[5:]
+            return (None, None, None, None, None, *_NoSecondOrder.apply(why, grads, *[h[3] for h in hyper]))
         grads = []
         vjp = None
         if kern._terms:
@@ -186,6 +193,134 @@ class _GramFn(torch.autograd.Function):
         return D
 
 
+def _no_second_order(hyper, dfields):
+    """ why the gradient of a Gram block with respect to `hyper` can not be differentiated again, or None """
+    if any(kind.startswith('bart_') for kind, _, _, _ in hyper):
+        return ('second derivatives through the BART kernel are not implemented: its alpha/beta derivatives are '
+                'first-order only')
+    if dfields != (-1, -1):
+        return ('second derivatives of the marginal likelihood with derivative observations are not implemented: they '
+                'would need the fourth derivative of the kernel core')
+    return None
+
+
+class _NoSecondOrder(torch.autograd.Function):
+    """ passes first-order gradients through; differentiating them raises NotImplementedError(why) (the inputs
+    `params` only attach the outputs to the graph, so that a second differentiation reaches this node) """
+
+    @staticmethod
+    def forward(ctx, why, values, *params):
+        ctx.why = why
+        return tuple(v.clone() for v in values)
+
+    @staticmethod
+    def backward(ctx, *grads):
+        raise NotImplementedError(ctx.why)
+
+
+def _gram_vjp_graph(kern, xd, yd, labels, G, hyper):
+    """ gradients with respect to the tensors of `hyper` of sum_ij G_ij K_ij, as differentiable functions of G and of
+    the hyperparameters: the per-factor contractions come from _GramVJPFn, their map to the user's tensors (the
+    1/scale of d/d log scale) stays in the torch graph """
+    params = [h[3] for h in hyper]
+    _, index = kern._descriptor(labels)
+    pos = {tf: i for i, tf in enumerate(index)}
+    vjp = _GramVJPFn.apply(kern, xd, yd, labels, G, *params).cpu()
+    grads = []
+    for kind, ti, fi, tensor in hyper:
+        if kind == 'amp':
+            g = vjp[pos[(ti, 0)], 0]
+        elif kind == 'scale':
+            g = vjp[pos[(ti, fi)], 1] / tensor.cpu()
+        elif kind == 'par1':
+            g = vjp[pos[(ti, fi)], 2]
+        else:  # pragma: no cover
+            raise NotImplementedError(kind)
+        grads.append(g.to(tensor.device, tensor.dtype).reshape(tensor.shape))
+    return grads
+
+
+class _GramVJPFn(torch.autograd.Function):
+    """ (G, theta) -> (nfactors, 3) per-factor contractions sum_ij G_ij dK_ij/d(amp, log scale, par1): the backward of
+    _GramFn as a differentiable function, for second derivatives.  Its backward, for a cotangent V on the contractions,
+    gives G the matrix sum_f V_f dK/dtheta_f (lgp_gram_iso_jvp) and the hyperparameters the second-order contraction
+    sum_ij G_ij d/dtheta (sum_f V_f dK_ij/dtheta_f) (lgp_gram_iso_hvp). """
+
+    @staticmethod
+    def forward(ctx, kern, xd, yd, labels, G, *params):
+        ctx.kern, ctx.xd, ctx.yd, ctx.labels = kern, xd, yd, labels
+        ctx.save_for_backward(G)
+        descs, _ = kern._descriptor(labels)
+        return _ops.gram_iso_vjp_general(descs, xd, yd, _ops.as_aligned(G.contiguous())).clone()
+
+    @staticmethod
+    def backward(ctx, V):
+        kern, xd, yd, labels = ctx.kern, ctx.xd, ctx.yd, ctx.labels
+        G, = ctx.saved_tensors
+        descs, index = kern._descriptor(labels)
+        tan = V.detach().cpu().numpy()
+        gG = _ops.gram_iso_jvp(descs, xd, yd, tan) if ctx.needs_input_grad[4] else None
+        hvp = _ops.gram_iso_hvp(descs, xd, yd, _ops.as_aligned(G.detach().contiguous()), tan).cpu()
+        pos = {tf: i for i, tf in enumerate(index)}
+        grads = []
+        for kind, ti, fi, tensor in kern._hyperparams():
+            if kind == 'amp':
+                g = hvp[pos[(ti, 0)], 0]
+            elif kind == 'scale':
+                g = hvp[pos[(ti, fi)], 1] / tensor.detach().cpu()
+            else:
+                g = hvp[pos[(ti, fi)], 2]
+            grads.append(g.to(tensor.device, tensor.dtype).reshape(tensor.shape))
+        return (None, None, None, None, gG, *grads)
+
+
+class _NegLogDensityGradFn(torch.autograd.Function):
+    """ (K, r, g) -> (g/2 (K^-1 - b b'), g b), b = K^-1 r: the backward of _NegLogDensityFn as a differentiable function,
+    for second derivatives.  K^-1 is the inverse of the jittered matrix that `dec` factors, as in the first-order
+    backward; K itself only routes the cotangent to the graph that built it.  For cotangents (W, w), W symmetrised:
+      K: g [-1/2 K^-1 W K^-1 + 1/2 (K^-1 W b b' + b b' W K^-1) - 1/2 (K^-1 w b' + b w' K^-1)]
+      r: g (K^-1 w - K^-1 W b)          g: 1/2 <W, K^-1 - b b'> + <w, b>
+    with K^-1 W K^-1 as two DMMA GEMMs, the second one on its lower triangle only. """
+
+    @staticmethod
+    def forward(ctx, dec, a, K, r, g):
+        b = dec._solve(a[:, None], True)[:, 0].contiguous()
+        low = dec.inverse_lower()
+        ctx.dec, ctx.low, ctx.b, ctx.g = dec, low, b, float(g)
+        return _ops.sym_expand_sub(low, b, scale=0.5 * float(g)), g * b
+
+    @staticmethod
+    def backward(ctx, W, w):
+        low, b, g = ctx.low, ctx.b, ctx.g
+        n = b.shape[0]
+        dev = b.device
+        Kinv = _ops.sym_expand_sub(low, None)
+        d = torch.zeros(n, dtype=f64, device=dev)    # K^-1 W b - K^-1 w
+        cot_g = torch.zeros((), dtype=f64, device=dev)
+        cotK = None
+        if W is not None:
+            W = _ops.as_aligned(0.5 * (W + W.T))
+            M1 = _ops.aligned_empty(n, n, dev)
+            _ops.dgemm(Kinv, W, M1, a_kmajor=True, b_kmajor=True, M=n, N=n, K=n, flags=_lib.GEMM_BETA0)
+            M2 = _ops.aligned_empty(n, n, dev)
+            _ops.dgemm(M1, Kinv, M2, a_kmajor=True, b_kmajor=True, M=n, N=n, K=n,
+                       flags=_lib.GEMM_BETA0 | _lib.GEMM_LOWER)
+            del M1
+            Wb = _ops.dgemv(W, b, torch.zeros(n, dtype=f64, device=dev))
+            _ops.dgemv(Kinv, Wb, d)
+            cot_g = cot_g + 0.5 * (_ops.symlower_dot(low, b, W)[0])
+            cotK = _ops.sym_expand_sub(M2, None, scale=-0.5 * g)
+            del M2
+        if w is not None:
+            w = w.contiguous()
+            _ops.dgemv(Kinv, w, d, alpha=-1.0)
+            cot_g = cot_g + torch.dot(w, b)
+        if cotK is None:
+            cotK = torch.zeros((n, n), dtype=f64, device=dev)
+        cotK += (0.5 * g) * (torch.outer(d, b) + torch.outer(b, d))
+        return None, None, cotK, -g * d, cot_g
+
+
 class _NegLogDensityFn(torch.autograd.Function):
     """ value = 1/2 (n log 2pi + log det K + r' K^-1 r)  (reference _decomp.py:484-488);
     backward: dvalue/dK = 1/2 (K^-1 - b b'), dvalue/dr = b, b = K^-1 r (reference _decomp.py:505-512). """
@@ -197,6 +332,7 @@ class _NegLogDensityFn(torch.autograd.Function):
         _timing.mark('decomp')
         ldq, a = dec.logdet_quad(r)
         ctx.dec, ctx.a = dec, a
+        ctx.save_for_backward(K, r)
         n = dec.n
         half = torch.tensor(0.5, dtype=f64, device=K.device)
         return half * (n * math.log(2 * math.pi) + 2 * ldq[0] + ldq[1])
@@ -204,6 +340,10 @@ class _NegLogDensityFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g):
         dec, a = ctx.dec, ctx.a
+        if torch.is_grad_enabled():   # create_graph: the gradient itself must be differentiable
+            K, r = ctx.saved_tensors
+            gK, gr = _NegLogDensityGradFn.apply(dec, a, K, r, g)
+            return gK if ctx.needs_input_grad[0] else None, gr if ctx.needs_input_grad[1] else None, None
         b = dec._solve(a[:, None], True)[:, 0]
         gK = gr = None
         if ctx.needs_input_grad[0]:
@@ -259,12 +399,22 @@ class _FusedNegLogMLFn(torch.autograd.Function):
         _timing.mark('decomp')
         ldq, a = dec.logdet_quad(r)
         ctx.kern, ctx.xd, ctx.labels, ctx.dec, ctx.a = kern, xd, labels, dec, a
+        ctx.save_for_backward(r)
         half = torch.tensor(0.5, dtype=f64, device=xd.device)
         return half * (dec.n * math.log(2 * math.pi) + 2 * ldq[0] + ldq[1])
 
     @staticmethod
     def backward(ctx, g):
         kern, xd, labels, dec, a = ctx.kern, ctx.xd, ctx.labels, ctx.dec, ctx.a
+        if torch.is_grad_enabled():
+            # create_graph: the same second order as the assembled route, through K built here (never on the
+            # first-order path) and the lower triangle of K^-1 kept by `dec`
+            r, = ctx.saved_tensors
+            hyper = kern._hyperparams()
+            K = _GramFn.apply(kern, xd, xd, labels, (-1, -1), *[h[3] for h in hyper])
+            gK, gr = _NegLogDensityGradFn.apply(dec, a, K, r, g)
+            grads = _gram_vjp_graph(kern, xd, xd, labels, gK, hyper) if hyper else []
+            return (None, None, None, gr if ctx.needs_input_grad[3] else None, None, *grads)
         b = dec._solve(a[:, None], True)[:, 0].contiguous()
         gr = g * b if ctx.needs_input_grad[3] else None
         hyper = kern._hyperparams()

@@ -14,7 +14,12 @@ without JAX:
   * the same scipy.optimize.minimize drivers are used: 'nograd' -> Nelder-Mead, 'gradient' -> BFGS,
     'fisher' -> dogleg with the Fisher information plus the prior precision as hessian (reference _fit.py:732-743,
     756-772): dK/dp comes from torch forward-mode AD through the Gram JVP kernel (lgp_gram_iso_jvp), the matrix
-    itself from Chol.minus_log_normal_density(fisher=True) (two blocked TRSMs per parameter on the DMMA path).
+    itself from Chol.minus_log_normal_density(fisher=True) (two blocked TRSMs per parameter on the DMMA path);
+    'hessian' -> trust-exact with the exact Hessian of the objective (torch.autograd.functional.hessian through the
+    twice-differentiable marginal likelihood).  trust-exact, not dogleg, because it accepts the indefinite Hessians
+    met away from the optimum, where dogleg requires positive definiteness;
+  * covariance: 'fisher', 'minhess', 'none', 'auto' as the reference, and 'hessian': the inverse of the exact Hessian
+    at the optimum (a RuntimeError if it is not positive definite).  'hessmod' is not implemented.
 """
 
 import math
@@ -24,7 +29,7 @@ import warnings
 
 import numpy
 import torch
-from scipy import optimize
+from scipy import linalg, optimize
 
 from . import _linalg
 from . import _timing
@@ -101,6 +106,10 @@ class empbayes_fit(Logger):
         Logger.__init__(self, verbosity)
         self.log('**** call lsqfitgp_b200.empbayes_fit ****')
         assert callable(gpfactory)
+        if method not in ('nograd', 'gradient', 'fisher', 'hessian'):
+            raise KeyError(method)
+        if covariance not in ('auto', 'fisher', 'minhess', 'hessian', 'none'):
+            raise KeyError(covariance)
         # `jit`: there is no tracing compiler here.  `forward`: the reference's forward mode materialises dK (n, n, k) with
         # jax.jacfwd and contracts it (_fit.py:679-685, _decomp.py:524-531); the same gradient is obtained here in ONE
         # reverse sweep by the fused VJP kernels (lgp_gram_iso_vjp / lgp_gram_bart_vjp), whatever the flag says: the
@@ -126,29 +135,34 @@ class empbayes_fit(Logger):
         self._timer = _timing.PhaseTimer()   # device time of the three phases of the reference's timer (_fit.py:410-442)
         self._hpunflat = hpunflat
 
+        def total_of(pt):
+            """ the objective as a torch function of the whitened parameters; starts the phase timer """
+            hp = hpunflat(pt)
+            gp = gpfactory(hp, **gpfactorykw)
+            args = data(hp, **gpfactorykw) if cachedargs is None else cachedargs
+            if not isinstance(args, tuple):
+                args = (args,)
+            self._timer.start()
+            try:
+                ml = gp.marginal_likelihood(*args, **mlkw)
+            except BaseException:
+                self._timer.stop()
+                raise
+            loss = -ml
+            prior = 1 / 2 * (len(pt) * math.log(2 * math.pi) + pt @ pt)
+            if isinstance(loss, torch.Tensor):
+                total = loss.cpu() + prior
+            else:
+                total = prior + loss
+            if additional_loss is not None:
+                extra = additional_loss(hp)
+                total = total + (extra.cpu() if isinstance(extra, torch.Tensor) else extra)
+            return total
+
         def objective(p, need_grad):
             pt = torch.tensor(numpy.asarray(p, dtype=float), dtype=f64, requires_grad=need_grad)
             with torch.set_grad_enabled(need_grad):
-                hp = hpunflat(pt)
-                gp = gpfactory(hp, **gpfactorykw)
-                args = data(hp, **gpfactorykw) if cachedargs is None else cachedargs
-                if not isinstance(args, tuple):
-                    args = (args,)
-                self._timer.start()
-                try:
-                    ml = gp.marginal_likelihood(*args, **mlkw)
-                except BaseException:
-                    self._timer.stop()
-                    raise
-                loss = -ml
-                prior = 1 / 2 * (len(pt) * math.log(2 * math.pi) + pt @ pt)
-                if isinstance(loss, torch.Tensor):
-                    total = loss.cpu() + prior
-                else:
-                    total = prior + loss
-                if additional_loss is not None:
-                    extra = additional_loss(hp)
-                    total = total + (extra.cpu() if isinstance(extra, torch.Tensor) else extra)
+                total = total_of(pt)
             if not need_grad:
                 self._timer.stop()
                 return float(total)
@@ -199,6 +213,17 @@ class empbayes_fit(Logger):
             fm = fm.cpu().numpy() if isinstance(fm, torch.Tensor) else numpy.asarray(fm)
             return fm + numpy.eye(k)
 
+        def hessian(p):
+            """ exact Hessian of the objective in p: torch.autograd.functional.hessian through the twice-differentiable
+            marginal likelihood (the GP term's second order runs lgp_gram_iso_hvp, lgp_gram_iso_jvp and DMMA GEMMs) """
+            self._ncalls['hess'] = self._ncalls.get('hess', 0) + 1
+            pt = torch.tensor(numpy.asarray(p, dtype=float), dtype=f64)
+            try:
+                H = torch.autograd.functional.hessian(total_of, pt)
+            finally:
+                self._timer.stop()
+            return H.numpy().astype(float)
+
         def fun(p):
             self._ncalls['fun'] += 1
             return objective(p, False)
@@ -220,11 +245,10 @@ class empbayes_fit(Logger):
         elif method == 'fisher':
             # dogleg requires positive definiteness; the Fisher matrix is p.s.d. and the prior precision is the identity
             minargs.update(hess=fisher, method='dogleg')
-        else:
-            raise KeyError(method)
+        elif method == 'hessian':
+            # trust-exact accepts the indefinite Hessians met away from the optimum, which dogleg does not
+            minargs.update(hess=hessian, method='trust-exact')
         self.log(f'method {method!r}', 2)
-        if covariance not in ('auto', 'fisher', 'minhess', 'none'):
-            raise KeyError(covariance)
 
         def callback(intermediate_result=None, *a):
             if self._verbosity >= 3:
@@ -274,7 +298,7 @@ class empbayes_fit(Logger):
             else:
                 self.log(msg)
 
-        cov = self._posterior_covariance(method, covariance, result, fisher)
+        cov = self._posterior_covariance(method, covariance, result, fisher, hessian)
         self._pcov_p = cov
         # the reference's totals line (_fit.py:775-794): device time per phase, the rest of the wall clock as 'other'
         times = dict(self._timer.totals)
@@ -488,7 +512,7 @@ class empbayes_fit(Logger):
             off += size
         return out
 
-    def _posterior_covariance(self, method, covariance, result, fisher_func):
+    def _posterior_covariance(self, method, covariance, result, fisher_func, hessian_func):
         """ reference _fit.py:808-845 """
         if covariance == 'auto':
             covariance = 'minhess' if (hasattr(result, 'hess_inv') or hasattr(result, 'hess')) else 'none'
@@ -496,6 +520,13 @@ class empbayes_fit(Logger):
             self.log('use fisher plus prior precision as precision', 2)
             prec = result.hess if method == 'fisher' else fisher_func(result.x)
             return _linalg.Chol(prec).ginv()
+        if covariance == 'hessian':
+            self.log('use the hessian at the optimum as precision', 2)
+            try:
+                cho = linalg.cho_factor(hessian_func(result.x), lower=True)
+            except numpy.linalg.LinAlgError:
+                raise RuntimeError('the hessian of the objective at the optimum is not positive definite') from None
+            return linalg.cho_solve(cho, numpy.eye(result.x.size))
         if covariance == 'minhess':
             if hasattr(result, 'hess_inv'):
                 hessinv = result.hess_inv

@@ -75,6 +75,8 @@ SIGNATURES = {
                                 _vp, _int, _vp]),
     'lgp_gram_iso_jvp': (_int, [_vp, ctypes.POINTER(Factor), _int, _int, _vp, _i64, _i64, _vp, _i64, _i64, c_double_p,
                                 _vp, _i64]),
+    'lgp_gram_iso_hvp': (_int, [_vp, ctypes.POINTER(Factor), _int, _int, _vp, _i64, _i64, _vp, _i64, _i64, _vp, _i64,
+                                _vp, _int, c_double_p, _vp]),
     'lgp_gram_iso_deriv': (_int, [_vp, ctypes.POINTER(Factor), _int, _int, _vp, _i64, _i64, _vp, _i64, _i64, _int, _int,
                                   _vp, _i64, _int]),
     'lgp_gram_iso_deriv_vjp': (_int, [_vp, ctypes.POINTER(Factor), _int, _int, _vp, _i64, _i64, _vp, _i64, _i64, _int,

@@ -141,6 +141,37 @@ def gram_iso_jvp(descs, x, y, tangent, out=None):
     return out
 
 
+def gram_iso_hvp(descs, x, y, G, tangent, b=None, symlower=False):
+    """ second-order contraction (lgp_gram_iso_hvp): (nfactors, 3) device tensor of
+    sum_ij G_ij d/d(amp, log scale, par1)_f of sum_g tangent_g dK_ij/dtheta_g; `tangent` as in gram_iso_jvp, G dense
+    (n, m), or with symlower=True the lower triangle of a symmetric G less b b' (the G of gram_iso_vjp) """
+    lib = _lib.load()
+    ndim, n = x.shape
+    x = x.contiguous() if x.stride(1) != 1 else x
+    y = x if symlower else (y.contiguous() if y.stride(1) != 1 else y)
+    m = y.shape[1]
+    assert G.shape == (n, m) and G.stride(1) == 1
+    tan = numpy.ascontiguousarray(numpy.asarray(tangent, dtype=numpy.float64).reshape(-1))
+    assert tan.size == 3 * len(descs)
+    buf = torch.empty(3 * len(descs), dtype=f64, device=x.device)
+    facs = make_factors(descs)
+    if b is not None:
+        b = b.contiguous()
+    check(lib.lgp_gram_iso_hvp(stream_ptr(), facs, len(descs), ndim, ptr(x), x.stride(0) if ndim else 0, n,
+                               ptr(y), y.stride(0) if ndim else 0, m, ptr(G), G.stride(0), ptr(b), 1 if symlower else 0,
+                               tan.ctypes.data_as(_lib.c_double_p), ptr(buf)), 'lgp_gram_iso_hvp')
+    return buf.reshape(len(descs), 3)
+
+
+def dgemv(P, x, y, alpha=1.0):
+    """ y += alpha P x in place (P: 2-D, unit column stride; x, y contiguous device vectors) """
+    lib = _lib.load()
+    assert P.stride(1) == 1 and x.is_contiguous() and y.is_contiguous()
+    check(lib.lgp_dgemv(stream_ptr(), 0, ptr(P), P.stride(0), P.shape[0], P.shape[1], ptr(x), ptr(y), float(alpha)),
+          'lgp_dgemv')
+    return y
+
+
 def gram_iso_deriv(descs, x, y, dx_field, dy_field, out=None, symmetric=False):
     """ derivative block d/dx_a d/dy_b k(x, y) (lgp_gram_iso_deriv): a = dx_field, b = dy_field field indices, -1 for
     no derivative on that argument; otherwise as gram_iso """
