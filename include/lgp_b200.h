@@ -135,6 +135,28 @@ int lgp_gram_iso_hvp(lgp_stream_t stream, const lgp_factor_t *factors, int nfact
                      int64_t ldx, int64_t n, const double *y, int64_t ldy, int64_t m, const double *G, int64_t ldg,
                      const double *b, int symlower, const double *tangent, double *out);
 
+/* Derivatives of the Gram build with respect to the points (what jax differentiating through the points of `gpfactory`
+ * gives the reference, src/lsqfitgp/_fit.py:687-702).  For a factor with field d in its dimmask,
+ *   dK/dx_{d,i} = amp c'(r2) 2 (u_{d,i} - v_{d,j}) / scale_x,   dK/dy_{d,j} = -amp c'(r2) 2 (u_{d,i} - v_{d,j}) / scale_y,
+ * u = (x - loc_x)/scale_x, v = (y - loc_y)/scale_y, with the product rule across the factors of a term; White and
+ * Constant contribute 0.  c' (u - v) is taken as 0 where u - v = 0, also where c' diverges at r = 0 (Maternp p = 0,
+ * Matern of low order, Cauchy alpha < 2): the exact value on the diagonal, where K(x_i, x_i) is constant.
+ *
+ * Reverse mode: gx[d*ldgx + i] = sum_j G_ij dK_ij/dx_{d,i}, gy[d*ldgy + j] = sum_i G_ij dK_ij/dy_{d,j}.  symlower = 0:
+ * G dense n x m (ldg), b_i b_j subtracted if b is not NULL; gx or gy may be NULL (not both).  symlower = 1: x == y,
+ * G_ij = w_ij (G[i][j] - b_i b_j) read from the LOWER triangle only, w = 2 off the diagonal, as in lgp_gram_iso_vjp;
+ * gx then receives the total derivative (both arguments) and gy must be NULL.  Outputs are device memory, zeroed by the
+ * call (fields outside every dimmask stay 0), accumulated with atomicAdd: the last bits may vary from run to run. */
+int lgp_gram_iso_xvjp(lgp_stream_t stream, const lgp_factor_t *factors, int nfactors, int ndim, const double *x,
+                      int64_t ldx, int64_t n, const double *y, int64_t ldy, int64_t m, const double *G, int64_t ldg,
+                      const double *b, int symlower, double *gx, int64_t ldgx, double *gy, int64_t ldgy);
+
+/* Forward mode: D[i][j] (+)= sum_d tx[d*ldtx + i] dK_ij/dx_{d,i} + ty[d*ldty + j] dK_ij/dy_{d,j}, tx and ty device
+ * (ndim, n) / (ndim, m) arrays, either may be NULL (a zero tangent).  accumulate = 1 adds to D, 0 overwrites it. */
+int lgp_gram_iso_xjvp(lgp_stream_t stream, const lgp_factor_t *factors, int nfactors, int ndim, const double *x,
+                      int64_t ldx, int64_t n, const double *y, int64_t ldy, int64_t m, const double *tx, int64_t ldtx,
+                      const double *ty, int64_t ldty, double *D_out, int64_t ldd, int accumulate);
+
 /* Derivative blocks: the covariance between first derivatives of the process, cov(d f(x)/d x_a, d f(y)/d y_b), with
  * a = dx_field, b = dy_field (field indices; -1 = no derivative on that argument, both -1 is LGP_ERR_BADARG).
  * Replaces the reference's jax derivatives of the kernel core behind addx(deriv=) and CrossKernel.linop('diff')

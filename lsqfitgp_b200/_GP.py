@@ -92,9 +92,10 @@ class _Cov(_Element):
 # ---------------------------------------------------------------------------------------------------------
 
 class _GramFn(torch.autograd.Function):
-    """ K = kernel(x, y) as a differentiable function of the kernel hyperparameters.
-    backward = lgp_gram_iso_vjp: sum_ij G_ij dK_ij/dtheta without materialising dK (reference: jax.vjp of the
-    Gram build, src/lsqfitgp/_fit.py:687-702). """
+    """ K = kernel(x, y) as a differentiable function of the kernel hyperparameters and of the points xd, yd.
+    backward = lgp_gram_iso_vjp: sum_ij G_ij dK_ij/dtheta without materialising dK, and lgp_gram_iso_xvjp for the points
+    (reference: jax.vjp of the Gram build, src/lsqfitgp/_fit.py:687-702).  BART terms depend on the points only through
+    integer bin indices: their contribution to the point gradient is 0, as under jax. """
 
     @staticmethod
     def forward(ctx, kern, xd, yd, labels, dfields, *params):
@@ -105,13 +106,33 @@ class _GramFn(torch.autograd.Function):
     def backward(ctx, G):
         kern, xd, yd, labels, dfields = ctx.kern, ctx.xd, ctx.yd, ctx.labels, ctx.dfields
         hyper = kern._hyperparams()
+        need_x, need_y = ctx.needs_input_grad[1], ctx.needs_input_grad[2]
+        if (need_x or need_y) and dfields != (-1, -1):
+            raise NotImplementedError(_NO_POINT_GRAD_DERIV)
         if torch.is_grad_enabled():   # create_graph: the gradient itself must be differentiable
             why = _no_second_order(hyper, dfields)
+            if why is None and (need_x or need_y):
+                why = _NO_POINT_SECOND_ORDER
             if why is None:
                 return (None, None, None, None, None, *_gram_vjp_graph(kern, xd, yd, labels, G, hyper))
             with torch.no_grad():
-                grads = _GramFn.backward(ctx, G.detach())[5:]
-            return (None, None, None, None, None, *_NoSecondOrder.apply(why, grads, *[h[3] for h in hyper]))
+                first = _GramFn.backward(ctx, G.detach())
+            gpts = [gp for gp in first[1:3] if gp is not None]
+            outs = _NoSecondOrder.apply(why, gpts + list(first[5:]), *[h[3] for h in hyper],
+                                        *((xd, yd) if gpts else ()))
+            it = iter(outs[:len(gpts)])
+            gx = next(it) if first[1] is not None else None
+            gy = next(it) if first[2] is not None else None
+            return (None, gx, gy, None, None, *outs[len(gpts):])
+        gx = gy = None
+        if need_x or need_y:
+            if kern._terms:
+                descs, _ = kern._descriptor(labels)
+                gx, gy = _ops.gram_iso_xvjp(descs, xd.detach(), yd.detach(), _ops.as_aligned(G.contiguous()),
+                                            need_x=need_x, need_y=need_y)
+            else:
+                gx = torch.zeros_like(xd) if need_x else None
+                gy = torch.zeros_like(yd) if need_y else None
         grads = []
         vjp = None
         if kern._terms:
@@ -138,15 +159,20 @@ class _GramFn(torch.autograd.Function):
             else:  # pragma: no cover
                 raise NotImplementedError(kind)
             grads.append(g.to(tensor.device, tensor.dtype).reshape(tensor.shape))
-        return (None, None, None, None, None, *grads)
+        return (None, gx, gy, None, None, *grads)
 
     @staticmethod
-    def jvp(ctx, _kern, _xd, _yd, _labels, _dfields, *tangents):
+    def jvp(ctx, _kern, tx, ty, _labels, _dfields, *tangents):
         """ forward mode (torch.autograd.forward_ad): dK along the tangent of the hyperparameters, one pass of
-        lgp_gram_iso_jvp; what jax.jacfwd of the Gram build gives the reference's Fisher path (_fit.py:676-683) """
+        lgp_gram_iso_jvp, plus that of the points tx, ty (lgp_gram_iso_xjvp, accumulated); what jax.jacfwd of the Gram
+        build gives the reference's Fisher path (_fit.py:676-683) """
         kern, xd, yd, labels, dfields = ctx.kern, ctx.xd, ctx.yd, ctx.labels, ctx.dfields
         hyper = kern._hyperparams()
         assert len(hyper) == len(tangents)
+        # points that are not on the dual level arrive with a materialised zero tangent: it contributes nothing
+        tx, ty = (None if t is None or not bool(torch.any(t != 0)) else t for t in (tx, ty))
+        if (tx is not None or ty is not None) and dfields != (-1, -1):
+            raise NotImplementedError(_NO_POINT_GRAD_DERIV)
         D = None
         if kern._terms:
             descs, index = kern._descriptor(labels)
@@ -168,6 +194,8 @@ class _GramFn(torch.autograd.Function):
                 D = _ops.gram_iso_deriv_jvp(descs, xd, yd, dfields[0], dfields[1], tan)
             else:
                 D = _ops.gram_iso_jvp(descs, xd, yd, tan)
+            if tx is not None or ty is not None:
+                _ops.gram_iso_xjvp(descs, xd.detach(), yd.detach(), tx, ty, D, accumulate=True)
         # BART terms: D += t_amp corr + t_alpha amp dcorr/dalpha + t_beta amp dcorr/dbeta, one kernel pass per term
         bart_tan = {}
         for (kind, ti, fi, tensor), t in zip(hyper, tangents):
@@ -191,6 +219,12 @@ class _GramFn(torch.autograd.Function):
         if D is None:
             D = torch.zeros(xd.shape[1], yd.shape[1], dtype=f64, device=xd.device)
         return D
+
+
+_NO_POINT_GRAD_DERIV = ('gradients with respect to the points through a derivative-observation block are not '
+                        'implemented: they need one more derivative order of the kernel')
+_NO_POINT_SECOND_ORDER = ('second derivatives with respect to the points are not implemented: the point derivatives '
+                          'of the Gram build are first-order only')
 
 
 def _no_second_order(hyper, dfields):
@@ -378,13 +412,15 @@ class _FusedNegLogMLFn(torch.autograd.Function):
     """ Gram -> Chol -> value in one node for the common case (one set of points, kernel-only covariance):
     the backward pass feeds the lower triangle of K^-1 and b = K^-1 r straight into the symmetric Gram-VJP
     kernel, so no dense n x n gradient matrix is ever formed (the two dK_vjp calls of the reference,
-    _decomp.py:505-509, collapse into one pass over the lower triangle). """
+    _decomp.py:505-509, collapse into one pass over the lower triangle).  The points xd are differentiable too: their
+    gradient is one more pass over the same triangle (lgp_gram_iso_xvjp). """
 
     @staticmethod
     def forward(ctx, kern, xd, labels, r, kw, *params):
         # the gradient will need K^-1: factorisation and inverse-from-factor in ONE library call, the inverse on a
         # persistent side stream (the latency-bound triangular solves below overlap its GEMMs)
-        side = _side_stream_for(torch.cuda.current_stream()) if any(ctx.needs_input_grad[5:]) else None
+        need_inverse = any(ctx.needs_input_grad[5:]) or ctx.needs_input_grad[1]
+        side = _side_stream_for(torch.cuda.current_stream()) if need_inverse else None
         # kernels of the fast family: the Gram build writes the equilibrated lower triangle and the Gershgorin partial
         # sums straight into the factor's storage (K itself is never materialised)
         descs, _ = kern._descriptor(labels)
@@ -406,6 +442,18 @@ class _FusedNegLogMLFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g):
         kern, xd, labels, dec, a = ctx.kern, ctx.xd, ctx.labels, ctx.dec, ctx.a
+        if torch.is_grad_enabled() and ctx.needs_input_grad[1]:
+            # create_graph with differentiable points: first order only
+            r, = ctx.saved_tensors
+            with torch.no_grad():
+                first = _FusedNegLogMLFn.backward(ctx, g.detach())
+            keep = [i for i in (1, 3) if first[i] is not None] + list(range(5, len(first)))
+            outs = _NoSecondOrder.apply(_NO_POINT_SECOND_ORDER, [first[i] for i in keep],
+                                        *[h[3] for h in kern._hyperparams()], xd, r)
+            res = [None] * len(first)
+            for i, o in zip(keep, outs):
+                res[i] = o
+            return tuple(res)
         if torch.is_grad_enabled():
             # create_graph: the same second order as the assembled route, through K built here (never on the
             # first-order path) and the lower triangle of K^-1 kept by `dec`
@@ -419,12 +467,18 @@ class _FusedNegLogMLFn(torch.autograd.Function):
         gr = g * b if ctx.needs_input_grad[3] else None
         hyper = kern._hyperparams()
         grads = []
-        if hyper:
+        gx = None
+        if hyper or ctx.needs_input_grad[1]:
             low = dec.inverse_lower()   # joins the side stream if the inverse was started in forward
             descs, index = kern._descriptor(labels)
-            vjp = (0.5 * _ops.gram_iso_vjp(descs, xd, low, b)).cpu()
+            if ctx.needs_input_grad[1]:
+                # the G of the hyperparameters' contraction: g/2 w_ij (K^-1 - b b')_ij on the lower triangle
+                gx = (0.5 * g) * _ops.gram_iso_xvjp(descs, xd.detach(), None, low, b, symlower=True)[0]
+            if hyper:
+                vjp = (0.5 * _ops.gram_iso_vjp(descs, xd, low, b)).cpu()
             del low
             dec._low = None   # 8 n^2 bytes: not needed again
+        if hyper:
             pos = {tf: i for i, tf in enumerate(index)}
             gc = g.cpu()
             for kind, ti, fi, tensor in hyper:
@@ -437,7 +491,7 @@ class _FusedNegLogMLFn(torch.autograd.Function):
                 else:  # pragma: no cover
                     raise NotImplementedError(kind)
                 grads.append((gc * v).to(tensor.device, tensor.dtype).reshape(tensor.shape))
-        return (None, None, None, gr, None, *grads)
+        return (None, gx, None, gr, None, *grads)
 
 
 class GP:
@@ -510,7 +564,12 @@ class GP:
             dfield = _Kernel.deriv_field(deriv, labels) if deriv.order <= 1 else None
             self._covfun._check_derivable(deriv, 0)
             self._dtype_names = names
-            xd = torch.from_numpy(numpy.ascontiguousarray(data)).to(dev)
+            if isinstance(data, torch.Tensor):
+                # points given as torch tensors stay on their autograd graph (and on a forward-mode dual level): the
+                # marginal likelihood is then differentiable with respect to them
+                xd = data.to(dev).contiguous()
+            else:
+                xd = torch.from_numpy(numpy.ascontiguousarray(data)).to(dev)
             self._elements[key] = _Points(labels, xd, tuple(shape), deriv, dfield)
 
     @_newself
@@ -668,7 +727,9 @@ class GP:
     # covariance blocks
     # ------------------------------------------------------------------------------------------------
     def _grad_mode(self):
-        return self._covfun is not None and torch.is_grad_enabled() and bool(self._covfun._hyperparams())
+        return self._covfun is not None and torch.is_grad_enabled() and (
+            bool(self._covfun._hyperparams()) or any(isinstance(e, _Points) and e.xd.requires_grad
+                                                     for e in self._elements.values()))
 
     def _makecovblock_points(self, xkey, ykey, out=None):
         x = self._elements[xkey]

@@ -267,8 +267,8 @@ class CrossKernel:
         if self._diff is not None:
             dfields = (deriv_field(self._diff[0], lx), deriv_field(self._diff[1], ly))
         dev = torch.device('cuda', torch.cuda.current_device())
-        xd = torch.from_numpy(numpy.ascontiguousarray(cx)).to(dev)
-        yd = torch.from_numpy(numpy.ascontiguousarray(cy)).to(dev)
+        xd, yd = (c.detach().to(dev).contiguous() if isinstance(c, torch.Tensor) else
+                  torch.from_numpy(numpy.ascontiguousarray(c)).to(dev) for c in (cx, cy))
         G = self._gram_device(xd, yd, lx, dfields=dfields).cpu().numpy()
         ix = numpy.broadcast_to(numpy.arange(cx.shape[1]).reshape(sx), shape)
         iy = numpy.broadcast_to(numpy.arange(cy.shape[1]).reshape(sy), shape)

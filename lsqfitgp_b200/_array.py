@@ -5,9 +5,14 @@ Mirrors the part of lsqfitgp's StructuredArray that the GP-fitting path relies o
 :555-564 _nd): one array per field, every leaf field (and every element of a shaped field) is
 one covariate dimension.  On the device the points are stored field-major, x[d, i], which is what
 the Gram kernels read (coalesced along i).
+
+Points may also be torch tensors, or dictionaries / StructuredArrays whose leaf fields are torch tensors (on the CPU
+or the GPU, possibly requiring grad): their columns stay torch tensors, so that gradients with respect to the points
+reach them (the reference differentiates through the points of `gpfactory` with jax, src/lsqfitgp/_fit.py:687-702).
 """
 
 import numpy
+import torch
 
 __all__ = ['StructuredArray', 'unstructured_to_structured', 'asarray']
 
@@ -44,7 +49,7 @@ class StructuredArray:
     def _init_from_dict(self, d):
         if not d:
             raise ValueError('empty dictionary')
-        arrays = {k: (v if isinstance(v, StructuredArray) else numpy.asarray(v)) for k, v in d.items()}
+        arrays = {k: (v if isinstance(v, (StructuredArray, torch.Tensor)) else numpy.asarray(v)) for k, v in d.items()}
         shape = None
         for k, v in arrays.items():
             s = v.shape
@@ -52,7 +57,8 @@ class StructuredArray:
         descr = []
         for k, v in arrays.items():
             sub = v.shape[len(shape):]
-            descr.append((k, v.dtype, sub) if sub else (k, v.dtype))
+            dt = _numpy_dtype(v)
+            descr.append((k, dt, sub) if sub else (k, dt))
         self._fields = arrays
         self.shape = shape
         self.dtype = numpy.dtype(descr)
@@ -128,7 +134,7 @@ class StructuredArray:
             if isinstance(col, StructuredArray):
                 out += [((name,) + lab if isinstance(lab, tuple) else (name, lab), c) for lab, c in col.leaf_columns()]
             else:
-                flat = numpy.asarray(col).reshape(n, -1)
+                flat = col.reshape(n, -1) if isinstance(col, torch.Tensor) else numpy.asarray(col).reshape(n, -1)
                 if flat.shape[1] == 1 and col.ndim == len(self.shape):
                     out.append((name, flat[:, 0]))
                 else:
@@ -137,6 +143,13 @@ class StructuredArray:
 
     def __repr__(self):
         return f'StructuredArray(shape={self.shape}, fields={list(self._fields)})'
+
+
+def _numpy_dtype(v):
+    """ numpy dtype of a field: a torch tensor's maps to the numpy dtype of the same name """
+    if isinstance(v, torch.Tensor):
+        return numpy.dtype(str(v.dtype).removeprefix('torch.'))
+    return v.dtype
 
 
 def _common_prefix(a, b):
@@ -162,8 +175,8 @@ def unstructured_to_structured(arr, dtype=None, names=None, **_):
 
 
 def asarray(x):
-    """ numpy array, or StructuredArray for structured inputs """
-    if isinstance(x, StructuredArray):
+    """ numpy array, or StructuredArray for structured inputs; a torch tensor is returned as it is """
+    if isinstance(x, (StructuredArray, torch.Tensor)):
         return x
     if isinstance(x, dict):
         return StructuredArray(x)
@@ -179,14 +192,35 @@ def asarray(x):
     return x
 
 
+_REAL_INT = (torch.bool, torch.uint8, torch.int8, torch.int16, torch.int32, torch.int64)
+
+
+def _check_tensor_dtype(t):
+    if not (t.dtype.is_floating_point or t.dtype in _REAL_INT):
+        raise TypeError(f'points have non-real dtype {t.dtype!r}')
+
+
 def columns_of(x):
-    """ (labels, (ndim, n) float64 numpy array, shape) of an array-like of points """
+    """ (labels, (ndim, n) float64 array, shape) of an array-like of points.  The array is numpy, or a torch tensor
+    (on the device of the first tensor column) when the points or any of their fields are torch tensors: built with
+    torch operations, it stays on the autograd graph of the points. """
     x = asarray(x)
     if isinstance(x, StructuredArray):
         cols = x.leaf_columns()
         labels = [c[0] for c in cols]
+        tensors = [c[1] for c in cols if isinstance(c[1], torch.Tensor)]
+        if tensors:
+            dev = tensors[0].device
+            for t in tensors:
+                _check_tensor_dtype(t)
+            data = torch.stack([c[1].to(dev, torch.float64) if isinstance(c[1], torch.Tensor) else
+                                torch.as_tensor(numpy.asarray(c[1], dtype=numpy.float64), device=dev) for c in cols])
+            return labels, data, x.shape
         data = numpy.stack([numpy.asarray(c[1], dtype=numpy.float64) for c in cols]) if cols else numpy.empty((0, x.size))
         return labels, data, x.shape
+    if isinstance(x, torch.Tensor):
+        _check_tensor_dtype(x)
+        return [None], x.reshape(1, -1).to(torch.float64), tuple(x.shape)
     if not (numpy.issubdtype(x.dtype, numpy.number) or x.dtype == bool):
         raise TypeError(f'points have non-numerical dtype {x.dtype!r}')
     return [None], x.reshape(1, -1).astype(numpy.float64), x.shape

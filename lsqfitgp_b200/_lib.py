@@ -77,6 +77,10 @@ SIGNATURES = {
                                 _vp, _i64]),
     'lgp_gram_iso_hvp': (_int, [_vp, ctypes.POINTER(Factor), _int, _int, _vp, _i64, _i64, _vp, _i64, _i64, _vp, _i64,
                                 _vp, _int, c_double_p, _vp]),
+    'lgp_gram_iso_xvjp': (_int, [_vp, ctypes.POINTER(Factor), _int, _int, _vp, _i64, _i64, _vp, _i64, _i64, _vp, _i64,
+                                 _vp, _int, _vp, _i64, _vp, _i64]),
+    'lgp_gram_iso_xjvp': (_int, [_vp, ctypes.POINTER(Factor), _int, _int, _vp, _i64, _i64, _vp, _i64, _i64, _vp, _i64,
+                                 _vp, _i64, _vp, _i64, _int]),
     'lgp_gram_iso_deriv': (_int, [_vp, ctypes.POINTER(Factor), _int, _int, _vp, _i64, _i64, _vp, _i64, _i64, _int, _int,
                                   _vp, _i64, _int]),
     'lgp_gram_iso_deriv_vjp': (_int, [_vp, ctypes.POINTER(Factor), _int, _int, _vp, _i64, _i64, _vp, _i64, _i64, _int,

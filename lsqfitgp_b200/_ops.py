@@ -163,6 +163,51 @@ def gram_iso_hvp(descs, x, y, G, tangent, b=None, symlower=False):
     return buf.reshape(len(descs), 3)
 
 
+def _ld(p):
+    """ leading dimension of a contiguous (ndim, n) point array (a one-row array may carry any stride) """
+    return p.stride(0) if p.shape[0] > 1 else p.shape[1]
+
+
+def gram_iso_xvjp(descs, x, y, G, b=None, symlower=False, need_x=True, need_y=True):
+    """ reverse-mode contraction with respect to the points (lgp_gram_iso_xvjp): (gx, gy), gx (ndim, n) =
+    sum_j G_ij dK_ij/dx_i, gy (ndim, m) = sum_i G_ij dK_ij/dy_j, G dense (n, m); with symlower=True (y is x) the lower
+    triangle of a symmetric G less b b' (the G of gram_iso_vjp), gx the total derivative and gy None.  A side not
+    `need`ed is None and not computed. """
+    lib = _lib.load()
+    ndim, n = x.shape
+    x = x.contiguous()
+    y = x if symlower else y.contiguous()
+    m = y.shape[1]
+    assert G.shape == (n, m) and G.stride(1) == 1
+    gx = torch.empty((ndim, n), dtype=f64, device=x.device) if (need_x or symlower) else None
+    gy = torch.empty((ndim, m), dtype=f64, device=x.device) if (need_y and not symlower) else None
+    facs = make_factors(descs)
+    if b is not None:
+        b = b.contiguous()
+    check(lib.lgp_gram_iso_xvjp(stream_ptr(), facs, len(descs), ndim, ptr(x), _ld(x), n, ptr(y), _ld(y), m,
+                                ptr(G), G.stride(0), ptr(b), 1 if symlower else 0, ptr(gx), n, ptr(gy), m),
+          'lgp_gram_iso_xvjp')
+    return gx, gy
+
+
+def gram_iso_xjvp(descs, x, y, tx, ty, out, accumulate=True):
+    """ forward-mode derivative with respect to the points (lgp_gram_iso_xjvp): out (n, m) (+)= sum_d tx[d, i]
+    dK_ij/dx_{d,i} + ty[d, j] dK_ij/dy_{d,j}; tx (ndim, n), ty (ndim, m) device tensors or None """
+    lib = _lib.load()
+    ndim, n = x.shape
+    m = y.shape[1]
+    x = x.contiguous()
+    y = y.contiguous()
+    tx = None if tx is None else tx.to(x.device, f64).contiguous()
+    ty = None if ty is None else ty.to(x.device, f64).contiguous()
+    assert out.shape == (n, m) and out.stride(1) == 1
+    facs = make_factors(descs)
+    check(lib.lgp_gram_iso_xjvp(stream_ptr(), facs, len(descs), ndim, ptr(x), _ld(x), n, ptr(y), _ld(y), m,
+                                ptr(tx), n, ptr(ty), m, ptr(out), out.stride(0), 1 if accumulate else 0),
+          'lgp_gram_iso_xjvp')
+    return out
+
+
 def dgemv(P, x, y, alpha=1.0):
     """ y += alpha P x in place (P: 2-D, unit column stride; x, y contiguous device vectors) """
     lib = _lib.load()
